@@ -50,7 +50,7 @@ WORKLOADS = {
                  desc="cfg1: 2-D radial SENSE-NUFFT A^H A apply, image 256x256, grid 512x512x2, 8 coils, 402 spokes x 512"),
     "cfg4": dict(N=(208, 208, 208), C=32, traj=("kooshball", 16384, 416), oversamp=2.0, kind="cg",
                  desc="cfg4: pics.py-style CG reconstruction, cfg3 geometry, 32 coils, sqrt-DCF row weights, lamda via "
-                      "cg(lamda=), 50 iterations; a step is one CG iteration (A^H A apply + fused BLAS-1 updates)"),
+                      "cg(lamda=), 50 iterations (--steps 50); a step is one CG iteration (A^H A apply + fused BLAS-1 updates)"),
     "cfg5": dict(N=(256, 256, 128), C=12, traj=("spirals", 128, 48, 2048), oversamp=2.0, kind="cfg5", full_coils=48,
                  desc="cfg5: stack-of-spirals SENSE-NUFFT 256x256x128 (grid 512x512x256), 128 x 48 spirals x 2048 samples "
                       "(M=12582912), 48 coils compressed to 12 virtual coils by a DenseMatrix cgemm; a step is one coil "
@@ -377,16 +377,18 @@ def run_ours(args):
         sync_all()
         lib.launch_count_reset()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        iters = 50
+        iters = steps
         e0.record()
         B.cg(AHA, b_h, xs, lamda=lam, tol=0.0, maxiter=iters, team=team)
         e1.record()
         sync_all()
         total_ms = e0.elapsed_time(e1)
         launches = lib.launch_count()
-        steps = iters + 1                                                          # 50 iterations + the initial residual apply
-        cg_info = {"iterations": iters, "seconds_per_solve": total_ms * 1e-3, "lamda": lam, "spectral_norm_estimate": nrm,
+        applies = iters + 1                                                        # the iterations + the initial residual apply
+        cg_info = {"iterations": iters, "applies": applies, "seconds_per_solve": total_ms * 1e-3, "lamda": lam,
+                   "spectral_norm_estimate": nrm,
                    "note": "timed region includes the H2D of b and x0 and the D2H of the solution (Backend.cg's contract)"}
+        outputs = {"solution": xs} if args.dump_outputs else None
     else:
         # ---- timed region: inputs resident in HBM --------------------------------------------------------
         lib.launch_count_reset()
@@ -397,6 +399,13 @@ def run_ours(args):
         sync_all()
         launches = lib.launch_count()
         total_ms = sum(a.elapsed_time(b) for a, b in ev)
+        applies = steps
+        outputs = None
+        if args.dump_outputs and rank == 0:
+            # what the last timed step handed back, read before anything else reuses the buffers
+            outputs = {"image": y_d.to_host()}
+            if extra is not None:
+                outputs["compressed_kspace"] = extra[2].to_host()
     # ---- per-kernel timing (outside the headline region): the same kernels, each bracketed by events -----------
     timer = KernelTimer(B, torch)
     ksteps = max(3, min(steps, 10))
@@ -439,8 +448,8 @@ def run_ours(args):
     if rank == 0:
         dom = kernels[0]
         line = {
-            "metric": "SENSE-NUFFT A^H A applies/sec", "value": steps / (total_ms * 1e-3), "unit": "applies/s",
-            "n_gpus": world, "steps": steps, "warmup": args.warmup, "ms_per_step": total_ms / steps,
+            "metric": "SENSE-NUFFT A^H A applies/sec", "value": applies / (total_ms * 1e-3), "unit": "applies/s",
+            "n_gpus": world, "steps": steps, "warmup": args.warmup, "ms_per_step": total_ms / applies,
             "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "complex64 (fp32 accumulate)",
             "data": "synthetic (seeded trajectory, rand64c image and unit-RSS coil maps)",
             "config": {"workload": wl["desc"],
@@ -464,7 +473,7 @@ def run_ours(args):
                          "frac_dram": dom["frac_dram"], "frac_replaced_call": dom["frac_replaced_call"],
                          "whole_apply": {"compulsory_bytes": int(sum(k["bytes"] for k in kernels)),
                                          "replaced_calls_bytes": int(sum(k["replaced_call_bytes"] for k in kernels)),
-                                         "frac": sum(k["bytes"] for k in kernels) / (total_ms / steps) / 1e6 / peak}},
+                                         "frac": sum(k["bytes"] for k in kernels) / (total_ms / applies) / 1e6 / peak}},
             "kernels": [{k: (round(v, 4) if isinstance(v, float) else v) for k, v in c.items()} for c in kernels],
             "clocks": clk,
             "setup": {"seconds": round(setup_s, 1), "peak_bytes_per_gpu": setup_bytes, "resident_bytes_per_gpu": resident_bytes},
@@ -488,12 +497,42 @@ def run_ours(args):
             line["cg"] = cg_info
         if check is not None:
             line["check"] = check
+        if outputs is not None:
+            line["outputs"] = dump_outputs(args.dump_outputs, outputs)
         if world == 1 and not args.no_cpu_baseline and args.workload in ("cfg3", "cfg4", "cfg1", "tiny"):
             line["cpu_baseline"] = cpu_baseline("cfg3" if args.workload == "cfg4" else args.workload, steps=1)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, arrays, budget=64 << 20):
+    """Writes each array as DIR/<name>.npy in float32 (complex values as (re, im) pairs), column-major order flattened.
+    An array larger than its share of `budget` bytes is replaced by a fixed sample: the elements at sorted indices
+    drawn without replacement by RandomState(0), written as <name>_sample.npy next to <name>_sample_index.npy
+    (float64), so that two builds run with the same arguments can be compared element for element."""
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // len(arrays) - 1024                  # room for the .npy headers
+    written = {}
+    for name, a in sorted(arrays.items()):
+        flat = np.asarray(a).ravel(order="F")
+        per = 8 if np.iscomplexobj(flat) else 4
+        idx = None
+        if flat.size * per > share:
+            keep = share // (per + 8)
+            idx = np.sort(np.random.RandomState(0).choice(flat.size, keep, replace=False))
+            flat, name = flat[idx], name + "_sample"
+        if np.iscomplexobj(flat):
+            out = np.ascontiguousarray(flat.astype(np.complex64)).view(np.float32).reshape(-1, 2)
+        else:
+            out = flat.astype(np.float32)
+        np.save(os.path.join(dirname, name + ".npy"), out)
+        written[name] = list(out.shape)
+        if idx is not None:
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.astype(np.float64))
+            written[name + "_index"] = [int(idx.size)]
+    return {"dir": dirname, "arrays": written}
 
 
 def power_norm(B, AHA, team, nvox, rs, iters=6):
@@ -809,6 +848,9 @@ def main():
     ap.add_argument("--check", action="store_true", help="correctness checks at the benchmarked size, outside the timed regions")
     ap.add_argument("--check-tree", action="store_true", help="with --check at N=1: also compare with the six-call recipe")
     ap.add_argument("--write-digest", action="store_true", help="with --check at N=1: store the image digest N>1 runs compare with")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all; "
+                         "larger outputs as a fixed seeded sample)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

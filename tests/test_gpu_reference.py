@@ -43,6 +43,13 @@ def B():
     return b200_reference_backend(0)
 
 
+@pytest.fixture(scope="module")
+def SB():
+    """Standalone build (no reference package involved)."""
+    from indigo_b200 import B200Backend
+    return B200Backend(0)
+
+
 def test_registered_with_the_reference_lookup(B, monkeypatch):
     indigo = reference()
     from indigo.backends import get_backend, available_backends
@@ -203,9 +210,10 @@ def test_hstack_values(B, stack, K, alpha, beta):
     np.testing.assert_allclose(vd.to_host(), alpha * (Hm.conj().T @ u) + beta * v, atol=1e-5)
 
 
-def test_int64_indices_split_into_column_blocks(B, monkeypatch):
+def test_int64_indices_split_into_column_blocks(SB, monkeypatch):
     """backend.py:549-550 keeps scipy's index dtype; cfg4's P on one GPU has 2.3 G columns and arrives with int64
     indices.  Here the block width is forced down so that a small int64 matrix takes the same path."""
+    B = SB
     rs = np.random.RandomState(4)
     M, N, K = 37, 101, 5
     A = (spp.random(M, N, density=0.2, random_state=rs, format='csr') +
@@ -235,9 +243,10 @@ def test_int64_indices_split_into_column_blocks(B, monkeypatch):
     assert abs(Ad._row_frac - frac) < 1e-12 and abs(Ad._col_frac - np.count_nonzero(np.bincount(A.indices, minlength=N)) / N) < 1e-12
 
 
-def test_dia_matrix_with_scipy_chosen_width(B):
+def test_dia_matrix_with_scipy_chosen_width(SB):
     """np.py:129-136 accepts whatever width scipy gives dia.data: todia() of a matrix with an empty last column is
     narrower than k, diags() with positive offsets on a wide matrix can be wider than the row count."""
+    B = SB
     rs = np.random.RandomState(9)
     A1 = spp.csr_matrix(np.array([[1, 2, 0, 0], [0, 3, 4, 0], [0, 0, 5, 0], [0, 0, 0, 0]], dtype=C64)).todia()
     assert A1.data.shape[1] < A1.shape[1]
