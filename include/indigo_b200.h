@@ -344,6 +344,26 @@ int ib200_sense_ifft_combine(ib200_sense_plan plan, void *stream, void *img_out,
 int ib200_sense_pass(ib200_sense_plan plan, void *stream, int which, void *grid_il, const void *img,
                      void *img_out, const void *pf, float alpha_re, float alpha_im, float beta_re, float beta_im);
 
+/* ------------------------------------------------------------------ Toeplitz normal operator
+ * A^H A of a SENSE operator as a zero-padded convolution (indigo_b200.fused.toeplitz_normal):
+ *   T x = s^2 * sum_c conj(S_c) .* crop( IFFT_L( K .* FFT_L( pad_L(S_c .* x) ) ) )
+ * on a plan created with oN = L (the padded grid, ib200_sense_plan_create) and pf = maps (no apodisation,
+ * no centring phase), without support windows.  One apply is five launches:
+ *   ib200_sense_pass 0 -> [1] -> ib200_sense_toeplitz_pass -> [4] -> ib200_sense_pass 5 (alpha = s^2 * alpha)
+ * (the bracketed y passes only when L[2] > 1).
+ *   ib200_sense_toeplitz_pass: on the last transformed axis (z, or y when L[2] == 1) loads the image window of
+ *     every line, transforms it forward, multiplies by kernel[pos * plane + point] (real float32, plane = L0*L1
+ *     points, or L0 when L[2] == 1; kernel is laid out like one coil of the grid, z slowest), and runs the first
+ *     inverse pass on it, storing the image window in the state ib200_sense_pass 3 leaves.  Lengths up to 512.
+ *   ib200_toeplitz_psf: psf[j] = (p(d) + conj p(-d)) / 2 for the circular lag d = j (mod L) per axis, with
+ *     p(d) = img[d + L/2] (column-major L0 x L1 x L2 complex64 images, x fastest; img != psf).
+ *   ib200_toeplitz_kernel: kernel[i] = scale * Re spectrum[i] for n points (spectrum = ib200_fft_exec of psf,
+ *     scale = 1 / prod(L)).
+ * None synchronises. */
+int ib200_sense_toeplitz_pass(ib200_sense_plan plan, void *stream, void *grid_il, const float *kernel);
+int ib200_toeplitz_psf(void *stream, const int64_t L[3], const void *img, void *psf);
+int ib200_toeplitz_kernel(void *stream, int64_t n, const void *spectrum, float scale, float *kernel);
+
 /* ------------------------------------------------------------------ operator construction on the device
  * Setup-time replacements for the host construction of the two sparse factors
  * of the -O3 SENSE tree (indigo/interp.py:19-80 + scipy COO->CSR + the -O2

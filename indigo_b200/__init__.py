@@ -9,7 +9,7 @@ Importing this package does not touch CUDA; the shared library is loaded (and
 its absence reported, loudly) when a backend is constructed.
 """
 __all__ = ["B200Backend", "get_backend", "register", "sense_operator", "sense_operator_fused", "normal_operator",
-           "CoilTeam"]
+           "toeplitz_normal", "CoilTeam"]
 
 
 def __getattr__(name):
@@ -22,6 +22,9 @@ def __getattr__(name):
     if name == "sense_operator_fused":
         from .fused import sense_operator_fused
         return sense_operator_fused
+    if name == "toeplitz_normal":
+        from .fused import toeplitz_normal
+        return toeplitz_normal
     if name == "CoilTeam":
         from .team import CoilTeam
         return CoilTeam

@@ -83,6 +83,9 @@ SIGNATURES = {
     "ib200_sense_expand_fft": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "ib200_sense_ifft_combine": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _f, _f]),
     "ib200_sense_pass": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _f, _f, _f, _f]),
+    "ib200_sense_toeplitz_pass": (_i, [_vp, _vp, _vp, _vp]),
+    "ib200_toeplitz_psf": (_i, [_vp, POINTER(_i64), _vp, _vp]),
+    "ib200_toeplitz_kernel": (_i, [_vp, _i64, _vp, _f, _vp]),
     "ib200_cgemm": (_i, [_vp, _i, _i64, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_csymm": (_i, [_vp, _i, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_cgemm_mode": (_i, [_i]),

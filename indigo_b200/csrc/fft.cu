@@ -274,6 +274,75 @@ static int try_pk_pass(cudaStream_t s, const IlPassArgs &a, int n, const FftStag
     return 0;
 }
 
+// Toeplitz convolution pass (fft_pkt_tile_body): persistent like fft_pkp_pass_kernel, same shared memory
+template <int N, int R0, int R1, int R2>
+__global__ void __launch_bounds__(kPkThreads, 2) fft_pkt_pass_kernel(const IlPassArgs a, int64_t ntiles,
+                                                                     const float *__restrict__ kern, int64_t kplane, int C) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float *bufA = reinterpret_cast<float *>(smem_raw);
+    c64 *raw = reinterpret_cast<c64 *>(bufA + pk_buf_floats(N));
+    c64 *stw = raw + (size_t)N * kSpecL;
+    const int tid = (int)threadIdx.x;
+    int64_t tile = blockIdx.x;
+    if (tile >= ntiles) return;
+    pkp_prefetch(a, tile, raw, tid, kPkThreads);
+    for (int i = tid; i < N; i += kPkThreads) stw[i] = a.tw[i];
+    while (tile >= 0) {
+        const int64_t next = tile + gridDim.x < ntiles ? tile + gridDim.x : -1;
+        pkp_wait();
+        __syncthreads();
+        fft_pkt_tile_body<N, R0, R1, R2, kPkThreads>(a, tile, next, bufA, raw, tid, kPkThreads, stw, kern, kplane, C);
+        tile = next;
+    }
+}
+
+// every stage of the Toeplitz pass runs in place at least once: all of them must stay within the 16 register pairs
+// per thread of the persistent pass (every length up to 512; the longer ones are never a Toeplitz grid)
+static constexpr int pk_inplace_pairs(int n, int r) { return ((kSpecL / 2 * (n / r) + kPkThreads - 1) / kPkThreads) * r; }
+static constexpr bool pkt_fits(int n, int r0, int r1, int r2) {
+    return pk_inplace_pairs(n, r0) <= 16 && pk_inplace_pairs(n, r1) <= 16 && (r2 <= 1 || pk_inplace_pairs(n, r2) <= 16);
+}
+
+template <int N, int R0, int R1, int R2>
+static int launch_pkt_pass(cudaStream_t s, const IlPassArgs &a, const float *kern, int64_t kplane, int C) {
+    const size_t smem = pk_buf_floats(N) * sizeof(float) + (size_t)N * kSpecL * sizeof(c64) + (size_t)N * sizeof(c64);
+    if constexpr (!pkt_fits(N, R0, R1, R2)) {
+        (void)s; (void)a; (void)kern; (void)kplane; (void)C; (void)smem;
+        set_error("Toeplitz pass: length %d does not fit the persistent packed pass", N);
+        return IB200_E_UNSUPPORTED;
+    } else {
+    static bool attr_done[64] = {false};
+    if ((int64_t)smem > smem_optin()) {
+        set_error("Toeplitz pass: length %d does not fit shared memory", N);
+        return IB200_E_UNSUPPORTED;
+    }
+    int dev = 0;
+    IB200_TRY(cudaGetDevice(&dev));
+    if (!attr_done[dev & 63]) {
+        IB200_TRY(cudaFuncSetAttribute(fft_pkt_pass_kernel<N, R0, R1, R2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_done[dev & 63] = true;
+    }
+    const int64_t ntiles = (a.inner / kSpecL) * a.outer;
+    int64_t blocks = (int64_t)sm_count() * 2;
+    if (blocks > ntiles) blocks = ntiles;
+    fft_pkt_pass_kernel<N, R0, R1, R2><<<(unsigned)blocks, kPkThreads, smem, s>>>(a, ntiles, kern, kplane, C);
+    IB200_LAUNCH_CHECK();
+    return 0;
+    }
+}
+
+static int run_pkt_pass(cudaStream_t s, const IlPassArgs &a, int n, const FftStages &st, const float *kern, int64_t kplane,
+                        int C) {
+    FftKernelArgs k;
+    k.n = n; k.st = st;
+#define IB200_PKT_PASS(nn, r0, r1, r2) \
+    if (fft_spec_matches(k, nn, r0, r1, r2)) return launch_pkt_pass<nn, r0, r1, r2>(s, a, kern, kplane, C);
+    IB200_FFT_SPEC_LIST(IB200_PKT_PASS)
+#undef IB200_PKT_PASS
+    set_error("Toeplitz pass needs an axis length with a specialised FFT (got %d)", n);
+    return IB200_E_UNSUPPORTED;
+}
+
 template <int N, int R0, int R1, int R2>
 __global__ void __launch_bounds__(kPkThreads, 2) sense_expand_pk_kernel(const SenseFftArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -670,6 +739,29 @@ int ib200_sense_pass(ib200_sense_plan plan, void *stream, int which, void *grid_
     const bool inverse = which >= 3;
     const int axis = (which == 1 || which == 4) ? 1 : 2;
     return sense_strided_pass(plan, s, (c64 *)grid_il, axis, inverse, inverse && axis == 2, !inverse && axis == 2);
+}
+
+/* Convolution pass of the Toeplitz normal operator on the last transformed axis (z, or y when oN[2] == 1): the
+ * forward transform of the input window, times kernel, then the first inverse pass; see include/indigo_b200.h. */
+int ib200_sense_toeplitz_pass(ib200_sense_plan plan, void *stream, void *grid_il, const float *kernel) {
+    IB200_RANGE("ib200_sense_toeplitz_pass");
+    IB200_REQUIRE(plan && grid_il && kernel, "null pointer");
+    IB200_REQUIRE(((uintptr_t)grid_il & 15) == 0, "grid must be 16-byte aligned");
+    IB200_REQUIRE(plan->win == nullptr, "the Toeplitz pass takes no support windows");
+    int rc = ensure_device_state(&plan->fft->d);
+    if (rc) return rc;
+    const int axis = plan->oN[2] > 1 ? 2 : 1;
+    IB200_REQUIRE(axis == 2 || plan->N[2] == 1, "2-D plans need a one-plane image");
+    const AxisPlan &ax = plan->fft->d.ax[axis];
+    const int64_t sy = plan->oN[0] * plan->C, sz = sy * plan->oN[1];
+    IlPassArgs a;
+    a.x = (c64 *)grid_il; a.tw = ax.tw_dev;
+    a.inner = axis == 2 ? sz : sy; a.outer = 1; a.outer_stride = a.inner * plan->oN[axis];
+    IB200_REQUIRE(a.inner % kSpecL == 0 && a.inner < (1LL << 32), "Toeplitz pass: grid slab must be a multiple of 16 lines");
+    a.pstride = (unsigned)a.inner;
+    a.in0 = a.out0 = (int)plan->off[axis];
+    a.in1 = a.out1 = (int)(plan->off[axis] + plan->N[axis]);
+    return run_pkt_pass(as_stream(stream), a, ax.n, ax.st, kernel, a.inner / plan->C, (int)plan->C);
 }
 
 }  // extern "C"

@@ -460,6 +460,65 @@ IB_HD void fft_pkp_tile_body(const IlPassArgs &a, int64_t tile, int64_t next, fl
     }
 }
 
+// ---- Toeplitz convolution pass (fused Toeplitz normal operator) ------------------------------------
+// One tile of the last transformed axis: forward transform of the input window, multiplication by the
+// real kernel K, re/im swap, forward transform again, store of the output window.  The stored lines are
+// the inverse transform in the swapped state the first inverse pass of ib200_sense_ifft_combine leaves
+// (the later inverse passes run forward transforms on swapped data), because K is real and commutes with
+// the conjugation.  K is indexed by position along the axis and grid point: kern[pos * kplane + (line of
+// the slab) / C].  Shared memory is that of the persistent pass (bufA + raw[] + twiddles): raw[] serves as
+// the second buffer of the stages, and the next tile is prefetched into it once the second transform has left
+// it, under the last stage (no stage runs in place: in-place stages, which would let the prefetch start
+// earlier, hold more registers than the 128 two CTAs per SM allow and spill).
+template <int N, int R0, int R1, int R2, int NT>
+IB_HD void fft_pkt_tile_body(const IlPassArgs &a, int64_t tile, int64_t next, float *bufA, c64 *raw, int tid, int nt,
+                             const c64 *tw, const float *kern, int64_t kplane, int C) {
+    constexpr bool THREE = R2 > 1;
+    float *bufB = reinterpret_cast<float *>(raw);
+    PkPrefCtx<false, false> c;
+    c.raw = raw; c.gout = const_cast<c64 *>(pkp_tile_base(a, tile)); c.tw = tw; c.pstride = a.pstride;
+    c.in0 = a.in0; c.inlen = (unsigned)(a.in1 - a.in0); c.out0 = a.out0; c.outlen = (unsigned)(a.out1 - a.out0);
+    pk_stage<N, R0, 1, true, false, NT>(c, nullptr, bufA, tid, nt);
+    IB_SYNC();                                                       // raw[] consumed, bufA complete
+    pk_stage<N, R1, R0, false, false, NT>(c, bufA, bufB, tid, nt);
+    IB_SYNC();
+    float *spec = bufB;                                              // spectrum: bufB (two stages) or bufA (three)
+    if (THREE) {
+        pk_stage<N, THREE ? R2 : R1, R0 * R1, false, false, NT>(c, bufB, bufA, tid, nt);
+        IB_SYNC();
+        spec = bufA;
+    }
+    // spectrum * K, swapped; the two lines of a pair may belong to two grid points (odd coil counts)
+    const unsigned s0 = (unsigned)((tile % (a.inner / kSpecL)) * kSpecL);     // a.inner < 2^32
+#pragma unroll 8
+    for (int i = tid; i < N * kPkPairs; i += (NT > 0 ? NT : nt)) {          // unrolled: the kernel loads overlap
+        const int pos = i / kPkPairs, lp = i % kPkPairs;
+        const unsigned p0 = (s0 + 2 * lp) / (unsigned)C, p1 = (s0 + 2 * lp + 1) / (unsigned)C;
+        const float *kr = kern + (int64_t)pos * kplane;
+#ifdef __CUDA_ARCH__
+        const pk2 kv = p_make(__ldg(kr + p0), __ldg(kr + p1));
+#else
+        const pk2 kv = p_make(kr[p0], kr[p1]);
+#endif
+        const cpk v = pk_lds<N>(spec, pos, lp);
+        pk_sts<N>(spec, pos, lp, k_mk(p_mul(v.y, kv), p_mul(v.x, kv)));
+    }
+    IB_SYNC();
+    if (THREE) {
+        pk_stage<N, R0, 1, false, false, NT>(c, bufA, bufB, tid, nt);
+        IB_SYNC();
+        pk_stage<N, R1, R0, false, false, NT>(c, bufB, bufA, tid, nt);
+        IB_SYNC();                                                   // raw[] free again
+        if (next >= 0) pkp_prefetch(a, next, raw, tid, nt);
+        pk_stage<N, THREE ? R2 : R1, R0 * R1, false, true, NT>(c, bufA, nullptr, tid, nt);
+    } else {
+        pk_stage<N, R0, 1, false, false, NT>(c, bufB, bufA, tid, nt);
+        IB_SYNC();                                                   // raw[] free again
+        if (next >= 0) pkp_prefetch(a, next, raw, tid, nt);
+        pk_stage<N, R1, R0, false, true, NT>(c, bufA, nullptr, tid, nt);
+    }
+}
+
 // ---- x passes of the fused SENSE transforms ------------------------------------------------------
 // Lines are coils (fft_il.cuh: sense_x_tile); a pair is two neighbouring coils of one image row, so
 // the coil count must be even.

@@ -90,6 +90,9 @@ class SenseDevice(object):
         lib, s = B._lib, B._stream
         N = tuple(int(v) for v in N)
         C = int(maps.shape[3])
+        # the construction's arguments, for operators derived from this one (toeplitz_normal)
+        self.coord, self.maps, self.weights = coord, maps, weights
+        self.oversamp, self.width, self.n = oversamp, width, n
         if C > 32:
             raise RuntimeError("fused SENSE path serves at most 32 coils per operator; shard or split the coils")
         self._plan = None
@@ -123,6 +126,7 @@ class SenseDevice(object):
         mod_at = _fftc_mod(self.oN)[cut].flatten(order='F')
         apod = rolloff3(omin, width, beta, N).flatten(order='F').astype(_C64)
         q = (mod_at * np.complex64(1)) * apod
+        self.q = q                                                     # (mod * apod) at the image voxels
         maps_f = maps.reshape((self.nvox, C), order='F').astype(_C64)
         self.pf = B.copy_array(np.ascontiguousarray(q[:, None] * maps_f).reshape(-1))
         # stored adjoint of G' with the grid points in (padded) tile-major order
@@ -458,10 +462,36 @@ def make_fused_classes(ops):
             d.samples_to_grid()
             d.ifft_combine(y, alpha, beta)
 
-    return FusedSenseNUFFT, FusedSenseNormal
+    class FusedSenseToeplitz(ops.Operator):
+        """T ~ A^H A : image -> image as a zero-padded FFT convolution (toeplitz_normal); no gridding."""
+
+        def __init__(self, backend, tdev, name='SENSE.toeplitz'):
+            ops.Operator.__init__(self, backend, name=name)
+            self._tdev = tdev
+
+        shape = property(lambda self: (self._tdev.nvox, self._tdev.nvox))
+        dtype = property(lambda self: _C64)
+
+        def _mem_usage(self, ncols=1):
+            return 0
+
+        def _eval(self, y, x, alpha=1, beta=0, forward=True, left=True):
+            if not left:
+                raise NotImplementedError("Right-multiplication not implemented for FusedSenseToeplitz.")
+            if x.shape[1] != 1:
+                raise ValueError("FusedSenseToeplitz takes one image at a time (got %d columns)" % x.shape[1])
+            self._tdev.apply(y, x, alpha, beta)
+
+    return FusedSenseNUFFT, FusedSenseNormal, FusedSenseToeplitz
 
 
 _cache = {}
+
+
+def _classes(ops):
+    if ops not in _cache:
+        _cache[ops] = make_fused_classes(ops)
+    return _cache[ops]
 
 
 def sense_operator_fused(B, N, coord, maps, oversamp=2.0, weights=None, width=3, n=128):
@@ -469,12 +499,170 @@ def sense_operator_fused(B, N, coord, maps, oversamp=2.0, weights=None, width=3,
     indigo_b200.sense.sense_operator).  Raises RuntimeError when the oversampled grid has no
     specialised FFT passes; callers then fall back to sense_operator_device / sense_operator."""
     from .sense import _ops_of
-    ops = _ops_of(B)
-    if ops not in _cache:
-        _cache[ops] = make_fused_classes(ops)
-    Fwd, _ = _cache[ops]
+    Fwd = _classes(_ops_of(B))[0]
     dev = SenseDevice(B, N, coord, maps, oversamp, weights, width, n)
     return Fwd(B, dev)
+
+
+# ---------------------------------------------------------------------------------------------------------
+# Toeplitz embedding of the normal operator.  The normal operator of a non-uniform DFT is Toeplitz:
+#     A^H A x = s^2 * sum_c conj(S_c) .* crop_N( IFFT_L( K .* FFT_L( pad_L(S_c .* x) ) ) ),
+#     K = Re FFT_L(p_sym) / prod(L),   p(d) ~ sum_m w_m^2 exp(+2 pi i kappa_m . d),  d in (-L/2, L/2)^3,
+# with L >= 2N - 1 per axis, so that every lag between two voxels of the image has its own grid point.  CG
+# applies A^H A fifty times per solve; this form has no gridding, no per-sample work and no k-space buffer in
+# the loop.  It is a different discretisation of the same model (DESIGN.md section 9): p comes from the gridded
+# adjoint the fused operator already has, on an image of L points per axis, so it carries the same Kaiser-Bessel
+# conventions, and s^2 is the least-squares fit of T to the gridded normal operator.
+TOEPLITZ_LENGTHS = (32, 52, 64, 104, 128, 192, 208, 256, 320, 384, 416, 448, 512, 640, 768, 832, 1024)
+TOEPLITZ_MAX = 512                  # longest axis of the convolution pass (ib200_sense_toeplitz_pass)
+TOEPLITZ_AUX_MAX = 832              # longest oversampled axis of the PSF's auxiliary operator: the fused passes of
+                                    # 1024-point axes do not fit shared memory (so 2-D 256^2 images are not served)
+TOEPLITZ_PROBE_SEED = 20            # seed of the probe image of the scale fit
+
+
+def toeplitz_grid(N, oversamp=2.0):
+    """Padded grid L of the Toeplitz embedding: per axis the smallest length L_d >= 2 N_d - 1 such that L_d and
+    the oversampled grid of an image of L_d points both have specialised passes that fit (1 for a one-point axis).
+    Raises RuntimeError when no such length exists."""
+    os3 = oversamp if isinstance(oversamp, tuple) else (oversamp,) * 3
+    L = []
+    for d, (nd, o) in enumerate(zip(N, os3)):
+        nd = int(nd)
+        if nd == 1:
+            L.append(1)
+            continue
+        ok = [l for l in TOEPLITZ_LENGTHS if l >= 2 * nd - 1 and l <= TOEPLITZ_MAX and int(l * o) in TOEPLITZ_LENGTHS
+              and int(l * o) <= TOEPLITZ_AUX_MAX]
+        if not ok:
+            raise RuntimeError("Toeplitz normal operator: no padded grid length with specialised passes for axis %d "
+                               "of %d points (oversampling %g)" % (d, nd, o))
+        L.append(ok[0])
+    if int(N[2]) > 1 and L[2] == 1:
+        raise RuntimeError("Toeplitz normal operator: bad image shape %s" % (tuple(N),))
+    return tuple(L)
+
+
+class ToeplitzDevice(object):
+    """Device-resident pieces of one Toeplitz normal operator: plan on the padded grid, kernel K, scale s^2."""
+
+    probe = None          # as SenseDevice.probe: label -> context manager around every pass of an apply
+
+    def __init__(self, dev, team=None):
+        from .sense import _ops_of
+        B = self.B = dev.B
+        lib, s = B._lib, B._stream
+        self.N, self.C, self.nvox = dev.N, dev.C, dev.nvox
+        self.L = L = toeplitz_grid(dev.N, dev.oversamp)
+        self.nL = nL = int(np.prod(L))
+        self.three = L[2] > 1
+        self._plan = None
+        # plan first: raises RuntimeError (unsupported) before anything large is built
+        plan = ctypes.c_void_p()
+        lib.sense_plan_create(ctypes.byref(plan), (ctypes.c_int64 * 3)(*self.N), (ctypes.c_int64 * 3)(*L), self.C)
+        self._plan = plan
+        # 1. PSF: adjoint of an auxiliary fused operator on an image of L points, applied to the k-space [w, 0]
+        #    (maps (1, 0): two coils keep it on the matrix-free construction)
+        aux_maps = np.zeros(L + (2,), dtype=_C64, order='F')
+        aux_maps[..., 0] = 1
+        aux = SenseDevice(B, L, dev.coord, aux_maps, dev.oversamp, dev.weights, dev.width, dev.n)
+        del aux_maps
+        ksp = np.zeros((aux.M * 2, 1), dtype=_C64, order='F')
+        ksp[:aux.M, 0] = 1 if dev.weights is None else np.asarray(dev.weights, dtype=np.float32).reshape(-1, order='F')
+        ksp_d = B.copy_array(ksp)
+        del ksp
+        img = B.empty_array((nL, 1), _C64, name='toeplitz.psf_image')
+        _classes(_ops_of(B))[0](B, aux)._eval(img, ksp_d, forward=False)
+        del ksp_d, aux
+        # 2. symmetrise into circular order, 3. L-point FFT, 4. K = Re(.) / prod(L)
+        psf = B.empty_array((nL, 1), _C64, name='toeplitz.psf')
+        lib.toeplitz_psf(s, (ctypes.c_int64 * 3)(*L), img.ptr, psf.ptr)
+        del img
+        fplan = ctypes.c_void_p()
+        lib.fft_plan_create(ctypes.byref(fplan), 3, (ctypes.c_int64 * 3)(*L), 1)
+        try:
+            lib.fft_exec(fplan, s, psf.ptr, psf.ptr, -1)
+            self.kernel = B.empty_array((nL,), np.dtype('float32'), name='toeplitz.K')
+            lib.toeplitz_kernel(s, nL, psf.ptr, 1.0 / nL, self.kernel.ptr)
+            lib.stream_sync(s)
+        finally:
+            lib.fft_plan_destroy(fplan)
+        del psf
+        self.grid = B.empty_array((nL * self.C,), _C64, name='toeplitz.grid[z][y][x][c]')
+        self.pf = B.copy_array(np.ascontiguousarray(dev.maps.reshape((self.nvox, self.C), order='F').astype(_C64)).reshape(-1))
+        # 5. scale: s^2 = Re<T1 v, N v> / ||T1 v||^2 with T1 = T at s = 1 and N the gridded normal operator, both
+        #    with the unit map on coil 0.  The fit depends on the trajectory only, not on the maps, so every coil
+        #    shard of an operator finds the same s^2 and the shards' T add up to the whole operator's T; with a
+        #    team the two sums are all-reduced as well, which makes s^2 bit-identical on every rank.
+        self.s2 = 1.0
+        rs = np.random.RandomState(TOEPLITZ_PROBE_SEED)
+        v = B.copy_array((rs.rand(self.nvox, 1) + 1j * rs.rand(self.nvox, 1)).astype(_C64, order='F'))
+        unit = np.zeros((self.nvox, self.C), dtype=_C64)
+        unit[:, 0] = 1
+        pf_t = B.copy_array(unit.reshape(-1))
+        unit[:, 0] = dev.q
+        pf_a = B.copy_array(unit.reshape(-1))
+        del unit
+        tv = B.empty_array((self.nvox, 1), _C64, name='toeplitz.probe.T')
+        av = B.empty_array((self.nvox, 1), _C64, name='toeplitz.probe.AHA')
+        self._passes(tv, v, pf_t, 1.0, 0.0)
+        lib.sense_expand_fft(dev._plan, s, dev.grid.ptr, v.ptr, pf_a.ptr)
+        dev.grid_to_samples()
+        dev.samples_to_grid()
+        lib.sense_ifft_combine(dev._plan, s, av.ptr, dev.grid.ptr, pf_a.ptr, 1.0, 0.0, 0.0, 0.0)
+        num, den = B.dot(tv, av), B.norm2(tv)
+        if team is not None:
+            num, den = team.allreduce(num), team.allreduce(den)
+        if not den > 0:
+            raise RuntimeError("Toeplitz normal operator: the trajectory gives an empty point-spread function")
+        self.s2 = float(num) / float(den)
+        del v, pf_t, pf_a, tv, av
+
+    def __del__(self):
+        try:
+            if getattr(self, '_plan', None):
+                self.B._lib.sense_plan_destroy(self._plan)
+        except Exception:
+            pass
+
+    def _step(self, label):
+        import contextlib
+        return self.probe(label) if self.probe is not None else contextlib.nullcontext()
+
+    def _passes(self, y, x, pf, alpha, beta):
+        lib, s, g = self.B._lib, self.B._stream, self.grid.ptr
+        a, b = complex(alpha) * self.s2, complex(beta)
+        with self._step("sense_expand_pk[x]"):
+            lib.sense_pass(self._plan, s, 0, g, x.ptr, None, pf.ptr, 1.0, 0.0, 0.0, 0.0)
+        if self.three:
+            with self._step("fft_pass[y fwd]"):
+                lib.sense_pass(self._plan, s, 1, g, None, None, None, 1.0, 0.0, 0.0, 0.0)
+        with self._step("toeplitz_pass[%s]" % ("z" if self.three else "y")):
+            lib.sense_toeplitz_pass(self._plan, s, g, self.kernel.ptr)
+        if self.three:
+            with self._step("fft_pass[y inv]"):
+                lib.sense_pass(self._plan, s, 4, g, None, None, None, 1.0, 0.0, 0.0, 0.0)
+        with self._step("sense_combine_pk[x]"):
+            lib.sense_pass(self._plan, s, 5, g, None, y.ptr, pf.ptr, a.real, a.imag, b.real, b.imag)
+
+    def apply(self, y, x, alpha=1.0, beta=0.0):
+        """y = alpha * T x + beta * y (beta == 0 never reads y)."""
+        self._passes(y, x, self.pf, alpha, beta)
+
+
+def toeplitz_normal(A, team=None):
+    """Toeplitz-embedded normal operator T ~ A^H A of a fused SENSE operator (from sense_operator_fused or
+    fuse_transform): an operator of the same family, shape (nvox, nvox), applied as a zero-padded FFT convolution
+    with a real kernel built once here.  It is not bit-parity with A^H A (DESIGN.md section 9): use it where the
+    gridded normal operator would go, e.g. B.cg(toeplitz_normal(A), A.H * y, x, lamda=...).  With a coil-sharded
+    operator pass the CoilTeam: every rank then uses the same scale.  Raises TypeError for any other operator and
+    RuntimeError when the padded grid has no specialised passes."""
+    dev = getattr(A, '_dev', None)
+    if not isinstance(dev, SenseDevice):
+        raise TypeError("toeplitz_normal takes a fused SENSE operator (sense_operator_fused / fuse_transform), got %s"
+                        % type(A).__name__)
+    from .sense import _ops_of
+    Toep = _classes(_ops_of(A._backend))[2]
+    return Toep(A._backend, ToeplitzDevice(dev, team), name=(getattr(A, '_name', '') or 'SENSE') + '.toeplitz')
 
 
 # ---------------------------------------------------------------------------------------------------------
