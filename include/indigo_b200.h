@@ -241,6 +241,21 @@ int ib200_kb_blocks_fill(void *stream, int64_t m, const void *records, const int
 int ib200_kb_blocks_apply(void *stream, int64_t ncols, int by, int bz, float alpha_re, float alpha_im, int nwork,
                           const int32_t *work, const void *entries, const void *Xil, int64_t xpitch, void *Yil,
                           int64_t ypitch, const int32_t *rowmap, int nsplit, const int32_t *split, void *scratch, int lanes);
+/* Pipe-Menon density compensation (csrc/dcf.cu; indigo_b200.sense.pipe_menon_dcf): w <- w / (I I^T w) with I the
+ * Kaiser-Bessel interpolation matrix, on the structures of the block gather above with 4x4x4 blocks and of
+ * ib200_kb_records (built without row weights, records in the sorted order with out = record position).
+ *   ib200_kb_density_spread: grid[rowmap[point]] = sum_e wz_e wy_e wx_e * w[out(e)], a real grid of prod(oN)
+ *     floats, for every point of a block that has a work item (points with rowmap < 0 are not written); scratch:
+ *     (work items of split blocks) * 64 floats.  Deterministic (fixed summation order, no atomics).
+ *   ib200_kb_density_update: per record q = inv_scale2 * sum_taps wz wy wx * grid[tap], then w[out] = w[out] / q, or
+ *     0 when q <= 0 or is not finite.  inv_scale2 = 1 / scale^2 for the scale the records carry, so that q is
+ *     (I I^T w) for the unscaled interpolation matrix.  residual (optional): 1 + ceil(m / 256) doubles of device
+ *     memory; residual[0] receives sum_r (q_r - 1)^2 in a fixed summation order.
+ * Neither synchronises. */
+int ib200_kb_density_spread(void *stream, int nwork, const int32_t *work, const void *entries, const float *w, float *grid,
+                            const int32_t *rowmap, int nsplit, const int32_t *split, float *scratch);
+int ib200_kb_density_update(void *stream, int64_t m, const void *records, const float *grid, const int64_t dims[3],
+                            float inv_scale2, float *w, double *residual);
 /* k-space support windows of a trajectory (fused SENSE recipe only).  Given the stored adjoint of the
  * gridding matrix in tile-major row order (rowptr[kp+1], rowmap[kp] from ib200_grid_tile_rank) the
  * grid columns are grouped into blocks of block[0] x block[1] points; for each block the hull [lo, hi)

@@ -9,14 +9,14 @@ Importing this package does not touch CUDA; the shared library is loaded (and
 its absence reported, loudly) when a backend is constructed.
 """
 __all__ = ["B200Backend", "get_backend", "register", "sense_operator", "sense_operator_fused", "normal_operator",
-           "toeplitz_normal", "CoilTeam"]
+           "pipe_menon_dcf", "toeplitz_normal", "CoilTeam"]
 
 
 def __getattr__(name):
     if name == "B200Backend":
         from .backend import B200Backend
         return B200Backend
-    if name in ("sense_operator", "normal_operator", "sqrt_dcf"):
+    if name in ("sense_operator", "normal_operator", "sqrt_dcf", "pipe_menon_dcf"):
         from . import sense
         return getattr(sense, name)
     if name == "sense_operator_fused":

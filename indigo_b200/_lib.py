@@ -61,6 +61,8 @@ SIGNATURES = {
     "ib200_kb_blocks_count": (_i, [_vp, _i64, _vp, POINTER(_i64), _i, _i, _vp, _i, _vp, _vp, POINTER(_i64)]),
     "ib200_kb_blocks_fill": (_i, [_vp, _i64, _vp, POINTER(_i64), _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "ib200_kb_blocks_apply": (_i, [_vp, _i64, _i, _i, _f, _f, _i, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _vp, _vp, _i]),
+    "ib200_kb_density_spread": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "ib200_kb_density_update": (_i, [_vp, _i64, _vp, _vp, POINTER(_i64), _f, _vp, _vp]),
     "ib200_grid_tile_rank2": (_i, [_vp, POINTER(_i64), POINTER(_i64), POINTER(_i64), _vp, POINTER(_i64)]),
     "ib200_grid_tile_rank": (_i, [_vp, POINTER(_i64), POINTER(_i64), _vp, _vp, POINTER(_i64)]),
     "ib200_csr_inspect": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, POINTER(_i64)]),

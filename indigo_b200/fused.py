@@ -130,14 +130,12 @@ class SenseDevice(object):
         maps_f = maps.reshape((self.nvox, C), order='F').astype(_C64)
         self.pf = B.copy_array(np.ascontiguousarray(q[:, None] * maps_f).reshape(-1))
         # stored adjoint of G' with the grid points in (padded) tile-major order
-        grid3, tile3 = (ctypes.c_int64 * 3)(*self.oN), (ctypes.c_int64 * 3)(*self.tile)
+        from .sense import tile_rowmap_device
+        grid3 = (ctypes.c_int64 * 3)(*self.oN)
         padded = ctypes.c_int64()
-        lib.grid_tile_rank(s, grid3, tile3, None, None, ctypes.byref(padded))
-        kp = self.kp = int(padded.value)
         i32 = np.dtype('int32')
-        colrank = B.empty_array((self.on,), i32)
-        self.rowmap = B.empty_array((kp,), i32, name='G.H.rowmap')
-        lib.grid_tile_rank(s, grid3, tile3, colrank.ptr, self.rowmap.ptr, ctypes.byref(padded))
+        kp, colrank, self.rowmap = tile_rowmap_device(B, self.oN, self.tile)
+        self.kp = kp
         self.t_ptr = self.t_ind = self.t_val = self.t_pk = None
         if not mf:
             self.t_ptr = B.empty_array((kp + 1,), i32, name='G.H.rowPtrs')
@@ -244,26 +242,14 @@ class SenseDevice(object):
         self.tiles = None
         shape = self._want_tiles()
         if self.real and self.kb is not None and shape:
+            from .sense import block_entries_device
             by, bz = shape
-            segb = max(1, int(self.tiles_seg_batches))
-            nblk = kp // 64 * (4 // by) * (4 // bz)
-            bptr = B.empty_array((nblk + 1,), i32, name='G.H.blocks.batchptr')
-            wptr = B.empty_array((nblk + 1,), i32, name='G.H.blocks.workptr')
-            tot = (ctypes.c_int64 * 5)()
-            lib.kb_blocks_count(s, self.M, self.kb.ptr, grid3, by, bz, self.rowmap.ptr, segb, bptr.ptr, wptr.ptr, tot)
-            nbat, nwork, nsplit, nslot = int(tot[1]), int(tot[2]), int(tot[3]), int(tot[4])
-            bb = int(lib.kb_blocks_batch_bytes(by, bz))
-            ent = B.empty_array((max(nbat, 1) * bb // 8,), np.dtype('int64'), name='G.H.blocks.entries')
-            work = B.empty_array((4 * max(nwork, 1),), i32, name='G.H.blocks.work')
-            split = B.empty_array((4 * max(nsplit, 1),), i32, name='G.H.blocks.split')
-            lib.kb_blocks_fill(s, self.M, self.kb.ptr, grid3, by, bz, segb, bptr.ptr, wptr.ptr, ent.ptr, work.ptr, split.ptr)
+            t = block_entries_device(B, self.M, self.kb, self.oN, self.rowmap, kp, shape, self.tiles_seg_batches)
             cl = 1
             while cl < min(C, 16) // 2:
                 cl *= 2
-            scratch = B.empty_array((max(nslot, 1) * 4 * by * bz * 2 * cl,), _C64, name='G.H.blocks.partial')
-            self.tiles = dict(ent=ent, work=work, nwork=nwork, split=split, nsplit=nsplit, scratch=scratch,
-                              batches=nbat, bytes=nbat * bb, shape=(by, bz))
-            del bptr, wptr
+            t['scratch'] = B.empty_array((max(t['nslot'], 1) * 4 * by * bz * 2 * cl,), _C64, name='G.H.blocks.partial')
+            self.tiles = t
         # x-run lists of the stored adjoint: one gather of a sample serves the four grid points of a tile row;
         # runs longer than run_long_thresh entries are cut into segments with their own lane groups
         self.runs = None

@@ -268,6 +268,155 @@ def kb_records_device(B, oN, coord, beta, weights=None, width=3, n=128, perm=Non
     return rec if flag.value == 0 else None
 
 
+def tile_rowmap_device(B, oN, tile):
+    """Tile-major row order of the oversampled grid (ib200_grid_tile_rank): (kp, colrank, rowmap) with kp the padded
+    point count, colrank[point] its tile-major row and rowmap[row] the grid point of a row (< 0: padding)."""
+    import ctypes
+    lib, s = B._lib, B._stream
+    grid3, tile3 = (ctypes.c_int64 * 3)(*oN), (ctypes.c_int64 * 3)(*tile)
+    padded = ctypes.c_int64()
+    lib.grid_tile_rank(s, grid3, tile3, None, None, ctypes.byref(padded))
+    kp = int(padded.value)
+    i32 = np.dtype('int32')
+    colrank = B.empty_array((int(np.prod(oN)),), i32)
+    rowmap = B.empty_array((kp,), i32, name='G.H.rowmap')
+    lib.grid_tile_rank(s, grid3, tile3, colrank.ptr, rowmap.ptr, ctypes.byref(padded))
+    return kp, colrank, rowmap
+
+
+def block_entries_device(B, m, records, oN, rowmap, kp, shape, seg_batches):
+    """Block entries of the matrix-free adjoint gridding (ib200_kb_blocks_count / _fill, csrc/kbblocks.cu) from the
+    separable records of m samples, for blocks of 4 x by x bz grid points (shape = (by, bz)) and the tile-major
+    rowmap of kp rows.  Returns dict(ent, work, nwork, split, nsplit, nslot, batches, bytes, shape); the caller
+    allocates the partial sums of the nslot work items of split blocks."""
+    import ctypes
+    lib, s = B._lib, B._stream
+    by, bz = shape
+    i32 = np.dtype('int32')
+    grid3 = (ctypes.c_int64 * 3)(*oN)
+    segb = max(1, int(seg_batches))
+    nblk = kp // 64 * (4 // by) * (4 // bz)
+    bptr = B.empty_array((nblk + 1,), i32, name='G.H.blocks.batchptr')
+    wptr = B.empty_array((nblk + 1,), i32, name='G.H.blocks.workptr')
+    tot = (ctypes.c_int64 * 5)()
+    lib.kb_blocks_count(s, m, records.ptr, grid3, by, bz, rowmap.ptr, segb, bptr.ptr, wptr.ptr, tot)
+    nbat, nwork, nsplit, nslot = int(tot[1]), int(tot[2]), int(tot[3]), int(tot[4])
+    bb = int(lib.kb_blocks_batch_bytes(by, bz))
+    ent = B.empty_array((max(nbat, 1) * bb // 8,), np.dtype('int64'), name='G.H.blocks.entries')
+    work = B.empty_array((4 * max(nwork, 1),), i32, name='G.H.blocks.work')
+    split = B.empty_array((4 * max(nsplit, 1),), i32, name='G.H.blocks.split')
+    lib.kb_blocks_fill(s, m, records.ptr, grid3, by, bz, segb, bptr.ptr, wptr.ptr, ent.ptr, work.ptr, split.ptr)
+    return dict(ent=ent, work=work, nwork=nwork, split=split, nsplit=nsplit, nslot=nslot, batches=nbat,
+                bytes=nbat * bb, shape=(by, bz))
+
+
+class DensityDevice(object):
+    """Device state of pipe_menon_dcf: the matrix-free construction of the fused operator without row weights
+    (sample order, separable records in sorted order with out = position, tile-major rowmap, support windows, 4x4x4
+    block entries), the real grid g = I^T w (prod(oN) float32, zeroed once) and the weights w in sorted order."""
+
+    probe = None          # as SenseDevice.probe: label -> context manager around each kernel of an iteration
+
+    def __init__(self, B, N, coord, oversamp=2.0, width=3, n=128):
+        import ctypes
+        from .fused import SenseDevice
+        coord = np.asarray(coord)
+        if not np.isfinite(coord).all():
+            raise ValueError("pipe_menon_dcf: the trajectory has non-finite coordinates")
+        self.B = B
+        lib, s = B._lib, B._stream
+        N = tuple(int(v) for v in N)
+        os3 = oversamp if isinstance(oversamp, tuple) else (oversamp,) * 3
+        oN = self.oN = tuple(int(a * o) for a, o in zip(N, os3))
+        omin = min(os3)
+        beta = np.pi * np.sqrt(((width * 2. / omin) * (omin - 0.5)) ** 2 - 0.8)       # as gridding_matrix_device
+        m = self.M = int(np.prod(coord.shape[1:]))
+        self.shape = tuple(coord.shape[1:])
+        self.grid3 = (ctypes.c_int64 * 3)(*oN)
+        self.perm, _ = sample_order_device(B, oN, coord, width, SenseDevice.sample_tile, SenseDevice.sample_super)
+        self.rec = kb_records_device(B, oN, coord, beta, None, width, n, perm=self.perm, out_sorted=True)
+        if self.rec is None:
+            raise RuntimeError("pipe_menon_dcf: no separable records for kernel width %g on the oversampled grid %s "
+                               "(they serve at most 6 taps per axis and a centring phase that is real up to a constant)"
+                               % (width, oN))
+        kp, colrank, rowmap = tile_rowmap_device(B, oN, SenseDevice.tile)
+        del colrank
+        i32 = np.dtype('int32')
+        win = B.empty_array((2 * oN[0] * oN[1],), i32, name='dcf.support')
+        self.rowmap = B.empty_array((kp,), i32, name='dcf.rowmap.support')
+        inside = ctypes.c_int64()
+        lib.kb_support_windows(s, m, self.rec.ptr, self.grid3, kp, rowmap.ptr, (ctypes.c_int64 * 3)(*SenseDevice.tile),
+                               win.ptr, self.rowmap.ptr, ctypes.byref(inside))
+        self.inside = int(inside.value)
+        del win, rowmap
+        self.tiles = block_entries_device(B, m, self.rec, oN, self.rowmap, kp, (4, 4), SenseDevice.tiles_seg_batches)
+        f32 = np.dtype('float32')
+        self.scratch = B.empty_array((max(self.tiles['nslot'], 1) * 64,), f32, name='dcf.partial')
+        self.g = B.zero_array((int(np.prod(oN)),), f32, name='dcf.grid')
+        self.w = B.copy_array(np.ones(m, dtype=np.float32))
+        self.resid = B.empty_array((1 + (m + 255) // 256,), np.dtype('float64'), name='dcf.residual')
+        # the records carry scale = 1/sqrt(prod oN) (float32) on z: the update divides q = scale^2 (I I^T w) by it
+        scl = float(np.float32(np.complex64(np.complex128(1.0) / np.sqrt(int(np.prod(oN)))).real))
+        self.inv_s2 = 1.0 / (scl * scl)
+
+    def _step(self, label):
+        import contextlib
+        return self.probe(label) if self.probe is not None else contextlib.nullcontext()
+
+    def iterate(self, residual=False):
+        """One iteration w <- w / (I I^T w); residual: also the sum of (I I^T w - 1)^2 into resid[0] (device)."""
+        lib, s, t = self.B._lib, self.B._stream, self.tiles
+        with self._step("kb_density_spread"):
+            lib.kb_density_spread(s, t['nwork'], t['work'].ptr, t['ent'].ptr, self.w.ptr, self.g.ptr, self.rowmap.ptr,
+                                  t['nsplit'], t['split'].ptr, self.scratch.ptr)
+        with self._step("kb_density_update"):
+            lib.kb_density_update(s, self.M, self.rec.ptr, self.g.ptr, self.grid3, self.inv_s2, self.w.ptr,
+                                  self.resid.ptr if residual else None)
+
+    def residual(self):
+        """||I I^T w - 1|| / sqrt(M) of the weights the last iterate(residual=True) started from (host read-back)."""
+        return float(np.sqrt(self.resid[0:1].to_host()[0] / self.M))
+
+    def weights(self):
+        """w in the caller's sample order, shaped like coord.shape[1:] (column-major)."""
+        out = np.empty(self.M, dtype=np.float32)
+        out[self.perm.to_host()] = self.w.to_host()
+        return out.reshape(self.shape, order='F')
+
+
+def pipe_menon_dcf(B, N, coord, oversamp=2.0, width=3, n=128, maxiter=30, history=None):
+    """Pipe-Menon density compensation of the trajectory `coord` (3, d1, d2, ...) for an image of shape N:
+        w_0 = 1,   w_{k+1} = w_k / (I I^T w_k),
+    I the Kaiser-Bessel interpolation matrix of the NUFFT on the oversampled grid (oversamp, width, n as for
+    sense_operator), so that the fixed point satisfies I I^T w = 1.  Unlike sqrt_dcf's |k|^(1/2) it is right for any
+    trajectory (stack of spirals, random, ...).  Both products run on the device with no matrix formed
+    (csrc/dcf.cu): I^T w on the 4x4x4 block entries of the matrix-free adjoint gridding, I g on the separable
+    records of the forward gridding, fused with the update.  No FFT plan is needed: grids the fused operator has no
+    passes for are served as well.
+
+    Returns float32 weights w shaped like coord.shape[1:] (samples in column-major order, as the operators take
+    them): weights=np.sqrt(w) feeds sense_operator_fused, sense_operator and fuse_transform trees as they are.
+    The result is bit-identical from run to run.  With `history` a list, the fixed-point residual
+    ||I I^T w_k - 1|| / sqrt(M) of the weights each iteration starts from (w_0 = 1 first) is appended to it, one
+    host read-back per iteration; without it the iterations issue no host synchronisation.
+    Under coil sharding every rank computes the same weights from the same trajectory; no collective is needed.
+    Raises ValueError for non-finite coordinates or maxiter < 1, RuntimeError when the separable records cannot be
+    built (kernels of more than 6 taps per axis, grids whose centring phase is not real up to a constant)."""
+    if int(maxiter) < 1:
+        raise ValueError("pipe_menon_dcf: maxiter must be at least 1, got %r" % (maxiter,))
+    coord = np.asarray(coord)
+    if int(np.prod(coord.shape[1:])) == 0:
+        return np.zeros(tuple(coord.shape[1:]), dtype=np.float32, order='F')
+    d = DensityDevice(B, N, coord, oversamp, width, n)
+    for _ in range(int(maxiter)):
+        d.iterate(residual=history is not None)
+        if history is not None:
+            history.append(d.residual())
+    w = d.weights()
+    del d                                   # device temporaries go with it
+    return w
+
+
 class _SixCallSense(object):
     """Mixin with the evaluation of the -O3 tree's six Backend calls (SURVEY.md section 3.1) on
     device-built operands; combined with the Operator base of B's family by sense_operator_device."""
