@@ -379,6 +379,32 @@ int ib200_sense_toeplitz_pass(ib200_sense_plan plan, void *stream, void *grid_il
 int ib200_toeplitz_psf(void *stream, const int64_t L[3], const void *img, void *psf);
 int ib200_toeplitz_kernel(void *stream, int64_t n, const void *spectrum, float scale, float *kernel);
 
+/* ------------------------------------------------------------------ orthonormal wavelets, l1-wavelet FISTA
+ * Separable periodized orthonormal wavelet transform W of a column-major dims[0] x dims[1] x dims[2] complex64
+ * image (DESIGN.md section 11).  h (host, lf doubles, lf = 2 or 8) is the low-pass filter; the high-pass filter is
+ * g[m] = (-1)^m h[lf-1-m].  Axes of one point are not transformed; every other axis must be divisible by
+ * 2^levels and at most 512 points long (longer: IB200_E_UNSUPPORTED).  Level j transforms the sub-box of extent
+ * dims[d] / 2^(j-1): an x pass, a y pass and a z pass, each in place on `work` (nvox complex64, device).
+ *   ib200_wavelet: y = alpha * W x + beta * y (inverse == 0) or alpha * W^H x + beta * y (inverse != 0);
+ *     beta == 0 never reads y.  work must not alias x or y.  A multi-level analysis ends with one elementwise
+ *     pass from work to y (its last wavelet pass covers only the coarse sub-box); a multi-level synthesis starts
+ *     with a device copy of x into work (its first pass covers only the coarse sub-box).
+ *   ib200_wavelet_fista_step: one prox-and-update step of FISTA (indigo_b200.wavelet.l1wavelet_recon), given
+ *     g = A^H A z:
+ *         x_new = W^H soft_thresh(W (z - step (g - b)))   (the coarse band of the last level is not thresholded)
+ *         z     = x_new + momentum[*counter] (x_new - x),   x = x_new,   *counter += 1
+ *     with soft_thresh(c) = c max(0, 1 - thresh / |c|).  The first analysis pass reads z, g and b, the last pass
+ *     of each analysis level thresholds on store and the last synthesis pass writes x and z.  stats (optional,
+ *     IB200_WAVELET_STATS doubles of device memory) receives stats[0] = ||x_new - x||^2, stats[1] = ||x_new||^2,
+ *     summed in a fixed order.  momentum and counter are device memory.
+ * Both are deterministic (no atomics) and neither synchronises. */
+#define IB200_WAVELET_STATS (2 + 2 * 4096)
+int ib200_wavelet(void *stream, const int64_t dims[3], int lf, const double *h, int levels, int inverse,
+                  float alpha_re, float alpha_im, float beta_re, float beta_im, const void *x, void *y, void *work);
+int ib200_wavelet_fista_step(void *stream, const int64_t dims[3], int lf, const double *h, int levels, float step,
+                             float thresh, const void *g, const void *b, void *z, void *x, void *work,
+                             const double *momentum, int *counter, double *stats);
+
 /* ------------------------------------------------------------------ operator construction on the device
  * Setup-time replacements for the host construction of the two sparse factors
  * of the -O3 SENSE tree (indigo/interp.py:19-80 + scipy COO->CSR + the -O2

@@ -88,6 +88,9 @@ SIGNATURES = {
     "ib200_sense_toeplitz_pass": (_i, [_vp, _vp, _vp, _vp]),
     "ib200_toeplitz_psf": (_i, [_vp, POINTER(_i64), _vp, _vp]),
     "ib200_toeplitz_kernel": (_i, [_vp, _i64, _vp, _f, _vp]),
+    "ib200_wavelet": (_i, [_vp, POINTER(_i64), _i, POINTER(c_double), _i, _i, _f, _f, _f, _f, _vp, _vp, _vp]),
+    "ib200_wavelet_fista_step": (_i, [_vp, POINTER(_i64), _i, POINTER(c_double), _i, _f, _f, _vp, _vp, _vp, _vp, _vp,
+                                      _vp, _vp, _vp]),
     "ib200_cgemm": (_i, [_vp, _i, _i64, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_csymm": (_i, [_vp, _i, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_cgemm_mode": (_i, [_i]),

@@ -67,6 +67,43 @@ def random_3d(rs, npts):
     return (rs.rand(3, npts, 1) - 0.5)
 
 
+# Modified 3-D Shepp-Logan ellipsoids (Kak and Slaney's table with Toft's contrasts), rotations about z only:
+#   intensity, semi-axes (a, b, c), centre (x0, y0, z0), rotation phi in degrees, on [-1, 1]^3.
+_PHANTOM = (
+    (1.0, .6900, .920, .810, 0.0, 0.0, 0.0, 0.0),
+    (-.8, .6624, .874, .780, 0.0, -.0184, 0.0, 0.0),
+    (-.2, .1100, .310, .220, .22, 0.0, 0.0, -18.0),
+    (-.2, .1600, .410, .280, -.22, 0.0, 0.0, 18.0),
+    (.1, .2100, .250, .410, 0.0, .35, -.15, 0.0),
+    (.1, .0460, .046, .050, 0.0, .1, .25, 0.0),
+    (.1, .0460, .046, .050, 0.0, -.1, .25, 0.0),
+    (.1, .0460, .023, .050, -.08, -.605, 0.0, 0.0),
+    (.1, .0230, .023, .020, 0.0, -.606, 0.0, 0.0),
+    (.1, .0230, .046, .020, .06, -.605, 0.0, 0.0),
+)
+
+
+def phantom(N):
+    """Deterministic piecewise-constant Shepp-Logan-like phantom of shape N = (N0, N1, N2), complex64, column-major
+    (x = axis 0 fastest).  Voxel i of an axis of n points sits at (2 i - n) / n in [-1, 1).  For N2 == 1 it is the
+    2-D phantom: the ellipses (a, b, x0, y0, phi) of the same table, with no z extent."""
+    N = tuple(int(v) for v in N)
+    ax = [(2.0 * np.arange(n) - n) / n for n in N]
+    X, Y, Z = np.meshgrid(ax[0], ax[1], ax[2], indexing='ij')
+    img = np.zeros(N, dtype=np.float64)
+    for amp, a, b, c, x0, y0, z0, phi in _PHANTOM:
+        if N[2] == 1 and z0 != 0.0:
+            continue
+        t = np.deg2rad(phi)
+        u = (X - x0) * np.cos(t) + (Y - y0) * np.sin(t)
+        v = -(X - x0) * np.sin(t) + (Y - y0) * np.cos(t)
+        r = (u / a) ** 2 + (v / b) ** 2
+        if N[2] > 1:
+            r = r + ((Z - z0) / c) ** 2
+        img[r <= 1.0] += amp
+    return np.asfortranarray(img.astype(np.complex64))
+
+
 def random_csr(rs, rows, cols, nnz_per_row):
     """cfg2: `nnz_per_row` distinct uniformly-random sorted columns per row, rand64c values.
     Returns (indptr int32, indices int32, data complex64)."""
