@@ -405,6 +405,26 @@ int ib200_wavelet_fista_step(void *stream, const int64_t dims[3], int lf, const 
                              float thresh, const void *g, const void *b, void *z, void *x, void *work,
                              const double *momentum, int *counter, double *stats);
 
+/* ------------------------------------------------------------------ ESPIRiT coil sensitivities (espirit.cu)
+ * DESIGN.md section 12.  All three are deterministic (fixed summation order, no atomics) and none synchronises.
+ * ib200_espirit_calib_gram: G = A^H A (n x n complex64, column-major, n = ncoils*k0*k1*k2) of the calibration
+ *   matrix A of the (w0, w1, w2, ncoils) column-major calibration k-space: one row per kernel position s with the
+ *   k0 x k1 x k2 patch inside the region, column (c, p) = p0 + k0 (p1 + k1 p2) + k0 k1 k2 c holding X_c(s + p).
+ *   fp32 accumulation; the upper triangle is computed and mirrored, the diagonal is real.
+ * ib200_espirit_lag_pass: out[o][x][i] = sum_{j < lags} in[o][j][i] * twiddle[x*lags + j], o < outer, x < n,
+ *   i < inner (one axis of the separable evaluation of the lag form).
+ * ib200_espirit_maps: per voxel (x, line), line = y + N1 z, M(x) = sum_j coef[line][j][c'][c] * twiddle0[x][j]
+ *   (the C x C matrix, row c, column c', coef laid out [line][lags0][ncoils][ncoils], c fastest); max_iter power
+ *   iterations from the all-ones vector, eig = the last norm, coil 0 rotated to real >= 0, zero where eig <= crop.
+ *   maps is (N0 N1 N2, ncoils) column-major complex64, eig N0 N1 N2 floats.  1 <= ncoils <= 32; the lag matrices
+ *   of one line must fit shared memory (lags0 * ncoils^2 * 8 bytes). */
+int ib200_espirit_calib_gram(void *stream, const int64_t w[3], const int64_t k[3], int ncoils, const void *calib,
+                             void *gram);
+int ib200_espirit_lag_pass(void *stream, int64_t outer, int lags, int n, int64_t inner, const void *twiddle,
+                           const void *in, void *out);
+int ib200_espirit_maps(void *stream, const int64_t N[3], int lags0, int ncoils, int max_iter, float crop,
+                       const void *twiddle0, const void *coef, void *maps, float *eig);
+
 /* ------------------------------------------------------------------ operator construction on the device
  * Setup-time replacements for the host construction of the two sparse factors
  * of the -O3 SENSE tree (indigo/interp.py:19-80 + scipy COO->CSR + the -O2

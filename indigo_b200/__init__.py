@@ -9,7 +9,7 @@ Importing this package does not touch CUDA; the shared library is loaded (and
 its absence reported, loudly) when a backend is constructed.
 """
 __all__ = ["B200Backend", "get_backend", "register", "sense_operator", "sense_operator_fused", "normal_operator",
-           "pipe_menon_dcf", "toeplitz_normal", "wavelet_operator", "l1wavelet_recon", "spectral_norm", "CoilTeam"]
+           "pipe_menon_dcf", "toeplitz_normal", "wavelet_operator", "l1wavelet_recon", "spectral_norm", "calibration_kspace", "espirit_maps", "CoilTeam"]
 
 
 def __getattr__(name):
@@ -28,6 +28,9 @@ def __getattr__(name):
     if name in ("wavelet_operator", "l1wavelet_recon", "spectral_norm"):
         from . import wavelet
         return getattr(wavelet, name)
+    if name in ("calibration_kspace", "espirit_maps"):
+        from . import espirit
+        return getattr(espirit, name)
     if name == "CoilTeam":
         from .team import CoilTeam
         return CoilTeam

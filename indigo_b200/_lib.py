@@ -91,6 +91,9 @@ SIGNATURES = {
     "ib200_wavelet": (_i, [_vp, POINTER(_i64), _i, POINTER(c_double), _i, _i, _f, _f, _f, _f, _vp, _vp, _vp]),
     "ib200_wavelet_fista_step": (_i, [_vp, POINTER(_i64), _i, POINTER(c_double), _i, _f, _f, _vp, _vp, _vp, _vp, _vp,
                                       _vp, _vp, _vp]),
+    "ib200_espirit_calib_gram": (_i, [_vp, POINTER(_i64), POINTER(_i64), _i, _vp, _vp]),
+    "ib200_espirit_lag_pass": (_i, [_vp, _i64, _i, _i, _i64, _vp, _vp, _vp]),
+    "ib200_espirit_maps": (_i, [_vp, POINTER(_i64), _i, _i, _i, _f, _vp, _vp, _vp, _vp]),
     "ib200_cgemm": (_i, [_vp, _i, _i64, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_csymm": (_i, [_vp, _i, _i64, _i64, _f, _f, _vp, _i64, _vp, _i64, _f, _f, _vp, _i64]),
     "ib200_cgemm_mode": (_i, [_i]),

@@ -25,6 +25,30 @@ def unit_rss_maps(rs, N, C):
     return np.asfortranarray((m / rss).astype(np.complex64))
 
 
+def birdcage_maps(N, C, r=1.5):
+    """Deterministic, smooth coil sensitivities (N0,N1,N2,C), complex64, column-major, unit root-sum-of-squares: the
+    birdcage model of sigpy.mri.birdcage_maps.  Coil c sits on a ring of radius r (image half-widths) around the z
+    axis with magnitude 1/distance and phase atan2(x', -y') - 2 pi c / C.  For 3-D images (N2 > 1) the coils form
+    rings of 8, stacked in z: coil c at angle 2 pi c / 8, height floor(c/8) - (ceil(C/8) - 1)/2, phase offset
+    -2 pi (c + floor(c/8)) / 8.  Voxel i of an axis of n points sits at (i - n/2) / (n/2)."""
+    N = tuple(int(v) for v in N)
+    C = int(C)
+    x, y, z = np.meshgrid(*[(np.arange(n) - n / 2.0) / (n / 2.0) for n in N], indexing='ij')
+    out = np.empty(N + (C,), dtype=np.complex128)
+    for c in range(C):
+        if N[2] > 1:
+            ang, cz = c * 2.0 * np.pi / 8, np.floor(c / 8) - 0.5 * (np.ceil(C / 8) - 1)
+            phs = -(c + np.floor(c / 8)) * 2.0 * np.pi / 8
+        else:
+            ang, cz, phs = c * 2.0 * np.pi / C, 0.0, -c * 2.0 * np.pi / C
+        xc, yc = x - r * np.cos(ang), y - r * np.sin(ang)
+        zc = z - cz if N[2] > 1 else 0.0
+        rr = np.sqrt(xc ** 2 + yc ** 2 + zc ** 2)
+        out[..., c] = np.exp(1j * (np.arctan2(xc, -yc) + phs)) / rr
+    out /= np.sqrt((np.abs(out) ** 2).sum(axis=3, keepdims=True))
+    return np.asfortranarray(out.astype(np.complex64))
+
+
 def radial_2d(nspokes=402, nread=512):
     """cfg1: in-plane radial, k = r*(cos t, sin t, 0), r in [-1/2,1/2), t_j = pi*j/nspokes.
     Returns coord (3, nread, nspokes) float64 (BART layout: ksp dims (1, nread, nspokes))."""
