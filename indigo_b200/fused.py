@@ -27,17 +27,18 @@ import ctypes
 
 import numpy as np
 
+from .sense import (GRID_TILE, SAMPLE_SUPER, SAMPLE_TILE, _mod_apod, block_entries_device, gridding_geometry,
+                    gridding_matrix_device, kb_records_device, sample_order_device, support_windows_device,
+                    tile_rowmap_device)
+
 _C64 = np.dtype('complex64')
 
 
 class SenseDevice(object):
     """Device-resident pieces shared by the fused nodes of one SENSE operator."""
 
-    tile = (4, 4, 4)
     allow_real = True          # use the real-weight packed kernels when the matrix values are real
     long_thresh = 512          # rows of G'^H with more entries than this get a whole CTA each
-    sample_tile = (8, 8, 8)    # samples (rows of G') are sorted by the grid tile of this size they fall into,
-    sample_super = (8, 8, 8)   # tiles grouped into super-tiles of this many tiles (64^3 points: L2-sized working set)
     # rows_per_group codes of ib200_ccsrmm_ilr (measured on cfg3, profiles/r01_s5_*): shared-memory staged
     # entries; one coil per lane for the long forward rows, two coils per lane for the short adjoint rows
     staged_fwd = -41
@@ -45,51 +46,24 @@ class SenseDevice(object):
     allow_separable = True     # forward gridding from 96-byte separable-weight records instead of stored entries
     allow_sorted_ksp = True    # keep k-space in tile-sorted sample order between the two gridding steps
     allow_runs = True          # adjoint gridding on merged x-runs of the stored adjoint (csrc/csrmm_runs.cu)
-    run_long_thresh = 1024     # runs with more entries than this are cut into segments of this length
+    run_long_thresh = None     # runs with more entries than this are cut into segments of this length (None: by size)
     allow_tiles = True         # adjoint gridding on block entries built from the separable records (csrc/kbblocks.cu)
     tiles_max_coils = 4        # whole 4x4x4 tiles up to this many coils (coil-sharded operators) ...
     blocks_max_coils = 64      # ... 4x2x2 blocks up to this many; the x-runs of the stored adjoint above
                                # (measured at cfg3, profiles/r02_blocks.md: 2 coils 1.15 / 2.77 ms, 4: 2.0 / 3.0,
                                #  8: 2.95 / 3.6, 16: 4.9 / 5.4 for blocks / x-runs)
     block_shape = None         # (by, bz) forced for every coil count (tests, tools/)
-    tiles_seg_batches = 256    # blocks with more batches (of 4 entries) than this are cut into work items of this length
+    tiles_seg_batches = None   # blocks of more batches (of 4 entries) than this are cut into work items (None: by size)
     tiles_lanes = 0            # lanes sharing the rows of a block (0: kernel default)
     matrix_free_setup = True   # build the matrix-free operator without ever forming the CSR matrix or its stored adjoint
-    keep_stored = False        # keep the CSR matrix and its stored adjoint after a matrix-free operator was built
     allow_windows = True       # k-space support windows: skip the grid outside the trajectory's support
     window_min_saving = 0.05   # ... when at least this fraction of the grid lies outside
 
     def __init__(self, B, N, coord, maps, oversamp=2.0, weights=None, width=3, n=128):
-        import os
-        from .sense import gridding_matrix_device, _fftc_mod, kb_records_device, _fftc_unit_phase
-        if os.environ.get("IB200_SAMPLE_SUPER"):                    # tuning knob: super-tile edge in tiles
-            self.sample_super = (int(os.environ["IB200_SAMPLE_SUPER"]),) * 3
-        if os.environ.get("IB200_SAMPLE_TILE"):                     # tuning knob: sample tile edge in grid points
-            self.sample_tile = (int(os.environ["IB200_SAMPLE_TILE"]),) * 3
-        if os.environ.get("IB200_TILES_MAXC"):                      # tuning knobs (tools/): tile-block adjoint gather
-            self.tiles_max_coils = int(os.environ["IB200_TILES_MAXC"])
-        if os.environ.get("IB200_BLOCKS_MAXC"):
-            self.blocks_max_coils = int(os.environ["IB200_BLOCKS_MAXC"])
-        if os.environ.get("IB200_BLOCKS_SHAPE"):
-            self.block_shape = tuple(int(v) for v in os.environ["IB200_BLOCKS_SHAPE"].split(","))
-        if os.environ.get("IB200_TILES_SEG"):
-            self.tiles_seg_batches = int(os.environ["IB200_TILES_SEG"])
-        if os.environ.get("IB200_RUN_LONG"):                        # tuning knob (tools/): run-length threshold
-            self.run_long_thresh = int(os.environ["IB200_RUN_LONG"])
-        elif int(np.prod(np.asarray(coord).shape[1:])) < (1 << 20) and type(self).run_long_thresh == 1024:
-            # small problems (cfg1: 0.2 M samples) are bound by the longest serial walk of one lane group, not by
-            # throughput: cut dense runs into shorter segments (r02 session 3: adjoint step 0.17 ms of a 0.37 ms apply)
-            self.run_long_thresh = 256
-        if (int(np.prod(np.asarray(coord).shape[1:])) < (1 << 20) and type(self).tiles_seg_batches == 256
-                and not os.environ.get("IB200_TILES_SEG")):
-            self.tiles_seg_batches = 32                             # the same for the block gather (r02 session 18: cfg1
-                                                                    # 0.141 -> 0.049 ms; 16 and 64 batches are slower)
-        from .kbmath import rolloff3
-
         self.B = B
-        lib, s = B._lib, B._stream
-        N = tuple(int(v) for v in N)
-        C = int(maps.shape[3])
+        lib = B._lib
+        geo = gridding_geometry(N, oversamp, width, n)
+        N, C = geo.N, int(maps.shape[3])
         # the construction's arguments, for operators derived from this one (toeplitz_normal)
         self.coord, self.maps, self.weights = coord, maps, weights
         self.oversamp, self.width, self.n = oversamp, width, n
@@ -98,162 +72,145 @@ class SenseDevice(object):
         self._plan = None
         # centring phase of G' that is real only up to a unit constant (2-D problems: -i on the two-point z axis): the
         # fused path holds conj(u) G', a real matrix, and applies u through alpha in the two gridding steps
-        os3 = oversamp if isinstance(oversamp, tuple) else (oversamp,) * 3
-        oN = tuple(int(a * o) for a, o in zip(N, os3))
-        omin = min(os3)
-        beta = np.pi * np.sqrt(((width * 2. / omin) * (omin - 0.5)) ** 2 - 0.8)       # as gridding_matrix_device
-        self.gphase = _fftc_unit_phase(oN) or 1.0
-        self.N, self.oN, self.C = N, oN, C
+        self.gphase = geo.u
+        self.N, self.oN, self.C = N, geo.oN, C
         self.M = int(np.prod(np.asarray(coord).shape[1:]))
-        self.nvox, self.on = int(np.prod(N)), int(np.prod(oN))
-        # matrix-free construction: sample order from the coordinates, windows and block entries from the separable
-        # records; the CSR matrix G' (10 GB at cfg3), its transposition and their sorts are never made.  Anything the
-        # matrix-free kernels do not serve (odd coil counts, complex centring phase, wide kernels, switches off) takes the
-        # construction on stored matrices below.
-        mf = bool(self.matrix_free_setup and self.allow_real and self.allow_separable and self.allow_sorted_ksp
-                  and self.allow_tiles and not self.keep_stored and self._want_tiles() is not None and self.M > 0)
-        self.G = None
-        if not mf:
-            self.G, oN_, omin_, beta_ = gridding_matrix_device(B, N, coord, oversamp, weights, width, n, unphase=self.gphase)
-            assert tuple(int(v) for v in oN_) == oN
-            self.nnz = int(self.G.values.size)
+        self.nvox, self.on = int(np.prod(N)), int(np.prod(self.oN))
+        # small problems (cfg1: 0.2 M samples) are bound by the longest serial walk of one lane group, not by
+        # throughput: dense runs and blocks are cut into shorter segments (r02 session 3: adjoint step 0.17 ms of a
+        # 0.37 ms apply; session 18: cfg1 block gather 0.141 -> 0.049 ms, 16 and 64 batches are slower)
+        small = self.M < (1 << 20)
+        if self.run_long_thresh is None:
+            self.run_long_thresh = 256 if small else 1024
+        if self.tiles_seg_batches is None:
+            self.tiles_seg_batches = 32 if small else 256
         # fused plan first: raises RuntimeError (unsupported) for grids without specialised passes
-        n3, on3 = (ctypes.c_int64 * 3)(*N), (ctypes.c_int64 * 3)(*self.oN)
         self._plan = ctypes.c_void_p()
-        lib.sense_plan_create(ctypes.byref(self._plan), n3, on3, C)
+        lib.sense_plan_create(ctypes.byref(self._plan), (ctypes.c_int64 * 3)(*N), (ctypes.c_int64 * 3)(*self.oN), C)
         # pf[voxel][coil] = (mod[zp] * apod)[voxel] * maps[voxel, coil]  (the factor P of pics.py:111-126)
-        cut = tuple(slice(a // 2 + int(np.ceil(-b / 2)), a // 2 + int(np.ceil(b / 2))) for a, b in zip(self.oN, N))
-        mod_at = _fftc_mod(self.oN)[cut].flatten(order='F')
-        apod = rolloff3(omin, width, beta, N).flatten(order='F').astype(_C64)
-        q = (mod_at * np.complex64(1)) * apod
-        self.q = q                                                     # (mod * apod) at the image voxels
+        self.q = _mod_apod(geo)[1]                                     # (mod * apod) at the image voxels
         maps_f = maps.reshape((self.nvox, C), order='F').astype(_C64)
-        self.pf = B.copy_array(np.ascontiguousarray(q[:, None] * maps_f).reshape(-1))
-        # stored adjoint of G' with the grid points in (padded) tile-major order
-        from .sense import tile_rowmap_device
-        grid3 = (ctypes.c_int64 * 3)(*self.oN)
-        padded = ctypes.c_int64()
-        i32 = np.dtype('int32')
-        kp, colrank, self.rowmap = tile_rowmap_device(B, self.oN, self.tile)
-        self.kp = kp
-        self.t_ptr = self.t_ind = self.t_val = self.t_pk = None
-        if not mf:
-            self.t_ptr = B.empty_array((kp + 1,), i32, name='G.H.rowPtrs')
-            self.t_ind = B.empty_array((max(self.nnz, 1),), i32, name='G.H.colInds')
-            self.t_val = B.empty_array((max(self.nnz, 1),), _C64, name='G.H.data')
-            work = B.empty_array((kp + 1,), i32)
-            lib.csr_transpose_conj(s, self.M, kp, self.nnz, self.G.values.ptr, self.G.colInds.ptr, self.G.rowPtrs.ptr,
-                                   self.t_val.ptr, self.t_ind.ptr, self.t_ptr.ptr, work.ptr, colrank.ptr)
-            del work
+        self.pf = B.copy_array(np.ascontiguousarray(self.q[:, None] * maps_f).reshape(-1))
+        # grid points in (padded) tile-major order: rows of the stored adjoint, blocks of the matrix-free one
+        self.kp, colrank, self.rowmap = tile_rowmap_device(B, self.oN)
+        self.G = self.t_ptr = self.t_ind = self.t_val = self.t_pk = self.longrows = None
+        self.g_map = self.g_ptr = self.g_pk = self.kb = self.pos = self.win = self.tiles = self.runs = None
+        self.real = self.ksp_sorted = False
+        self.nlong, self.support_fraction = 0, 1.0
+        # matrix-free construction unless the matrix-free kernels do not serve the operator (odd coil counts, complex
+        # centring phase, wide kernels, switches off); the records' kernel may still refuse a sample
+        mf = (self.matrix_free_setup and self.allow_real and self.allow_sorted_ksp and geo.separable
+              and self._want_tiles() is not None and self.M > 0)
+        if not (mf and self._build_matrix_free(geo, coord, weights)):
+            self._build_stored(geo, coord, weights, colrank)
         del colrank
+        # zero-initialised: with windows, parts of the grid are never written, and the separable gather
+        # multiplies its zero-weight taps (6th tap of on-grid samples) with whatever is there
+        self.grid = B.zero_array((self.on * C,), _C64, name='grid[z][y][x][c]')
+        self.ksp = B.empty_array((self.M * C,), _C64, name='ksp[m][c]')
+
+    def _build_matrix_free(self, geo, coord, weights):
+        """Sample order, separable records, windows and block entries, all from the coordinates: G' (10 GB at cfg3)
+        and its transposition are never made.  Returns False, keeping nothing, when the records cannot be built."""
+        B = self.B
+        lib, s = B._lib, B._stream
+        g_map, nnz = sample_order_device(B, geo, coord)
+        kb = kb_records_device(B, geo, coord, weights, perm=g_map, out_sorted=True)
+        if kb is None:
+            return False
+        self.g_map, self.nnz, self.kb = g_map, nnz, kb
+        self.real = self.ksp_sorted = True
+        self.pos = B.empty_array((max(self.M, 1),), np.dtype('int32'), name='G.sorted.position')
+        lib.invert_perm(s, self.M, g_map.ptr, self.pos.ptr)
+        bx = self._window_block_x()
+        if bx:
+            self._adopt_windows(*support_windows_device(B, self.M, kb, self.oN, self.kp, self.rowmap, bx), bx)
+        self._build_blocks()
+        return True
+
+    def _build_stored(self, geo, coord, weights, colrank):
+        """G' and its stored adjoint in tile-major row order, packed and sorted entries, records, long rows, windows
+        from the stored adjoint, then block entries or x-runs.  With block entries both gridding steps are matrix-free:
+        the stored matrices were only the source of the windows and are released (17 GB at cfg3)."""
+        B, C, M, kp = self.B, self.C, self.M, self.kp
+        lib, s = B._lib, B._stream
+        i32, pk = np.dtype('int32'), np.dtype('int64')          # pk: 8-byte (int32 column, float32 weight) records
+        self.G = gridding_matrix_device(B, self.N, coord, self.oversamp, weights, self.width, self.n,
+                                        unphase=self.gphase)[0]
+        nnz = self.nnz = int(self.G.values.size)
+        self.t_ptr = B.empty_array((kp + 1,), i32, name='G.H.rowPtrs')
+        self.t_ind = B.empty_array((max(nnz, 1),), i32, name='G.H.colInds')
+        self.t_val = B.empty_array((max(nnz, 1),), _C64, name='G.H.data')
+        work = B.empty_array((kp + 1,), i32)
+        lib.csr_transpose_conj(s, M, kp, nnz, self.G.values.ptr, self.G.colInds.ptr, self.G.rowPtrs.ptr,
+                               self.t_val.ptr, self.t_ind.ptr, self.t_ptr.ptr, work.ptr, colrank.ptr)
+        del work
         # real-weight packed entries (8 B instead of 12 B per stored entry, half the multiplies) when
         # the centring phase folded into G' is real, i.e. on every grid the fused path serves
-        self.real, self.kb, self.ksp_sorted, self.pos = False, None, False, None
-        if mf:
-            from .sense import sample_order_device
-            self.g_map, self.nnz = sample_order_device(B, self.oN, coord, width, self.sample_tile, self.sample_super)
-            self.kb = kb_records_device(B, self.oN, coord, beta, weights, width, n, perm=self.g_map, out_sorted=True)
-            if self.kb is not None:
-                self.real = self.ksp_sorted = True
-                self.pos = B.empty_array((max(self.M, 1),), i32, name='G.sorted.position')
-                lib.invert_perm(s, self.M, self.g_map.ptr, self.pos.ptr)
-                self.g_pk = self.g_ptr = None
-        elif self.nnz and self.allow_real:
-            pk = np.dtype('int64')                                     # 8-byte (int32 column, float32 weight) records
-            g_pk = B.zero_array((self.nnz + 2,), pk, name='G.packed')  # +2: the staged kernel copies 16-byte granules
+        if nnz and self.allow_real:
+            g_pk = B.zero_array((nnz + 2,), pk, name='G.packed')   # +2: the staged kernel copies 16-byte granules
             hmax = (ctypes.c_float * 2)()
-            lib.csr_pack_real(s, self.nnz, self.G.values.ptr, self.G.colInds.ptr, g_pk.ptr, hmax)
+            lib.csr_pack_real(s, nnz, self.G.values.ptr, self.G.colInds.ptr, g_pk.ptr, hmax)
             if hmax[1] <= 1e-8 * hmax[0]:
-                t_pk = B.zero_array((self.nnz + 2,), pk, name='G.H.packed')
-                lib.csr_pack_real(s, self.nnz, self.t_val.ptr, self.t_ind.ptr, t_pk.ptr, hmax)
-                self.t_pk, self.real = t_pk, True
-                self.t_val = self.t_ind = None                          # the complex copy of G'^H is not needed any more
+                self.t_pk = B.zero_array((nnz + 2,), pk, name='G.H.packed')
+                lib.csr_pack_real(s, nnz, self.t_val.ptr, self.t_ind.ptr, self.t_pk.ptr, hmax)
+                self.real = True
+                self.t_val = self.t_ind = None                  # the complex copy of G'^H is not needed any more
                 # samples sorted by the 8x8x8 grid tile they fall into, tiles grouped into 64^3 super-tiles: the
                 # samples one CTA sweeps share operand lines in all three dimensions (L1) and the CTAs in
                 # flight cover a compact block of the grid (L2)
-                stile = (ctypes.c_int64 * 3)(*self.sample_tile)
-                ssuper = (ctypes.c_int64 * 3)(*self.sample_super)
+                grid3 = (ctypes.c_int64 * 3)(*self.oN)
+                stile, ssuper = (ctypes.c_int64 * 3)(*SAMPLE_TILE), (ctypes.c_int64 * 3)(*SAMPLE_SUPER)
+                padded = ctypes.c_int64()
                 lib.grid_tile_rank2(s, grid3, stile, ssuper, None, ctypes.byref(padded))
-                nr8 = int(padded.value)
                 rank8 = B.empty_array((self.on,), i32)
                 lib.grid_tile_rank2(s, grid3, stile, ssuper, rank8.ptr, ctypes.byref(padded))
-                self.g_ptr = B.empty_array((self.M + 1,), i32, name='G.sorted.rowPtrs')
-                self.g_pk = B.zero_array((self.nnz + 2,), pk, name='G.sorted.packed')
-                self.g_map = B.empty_array((max(self.M, 1),), i32, name='G.sorted.rowmap')
-                lib.csr_permute_rows(s, self.M, self.nnz, self.G.rowPtrs.ptr, g_pk.ptr, rank8.ptr, nr8,
+                self.g_ptr = B.empty_array((M + 1,), i32, name='G.sorted.rowPtrs')
+                self.g_pk = B.zero_array((nnz + 2,), pk, name='G.sorted.packed')
+                self.g_map = B.empty_array((max(M, 1),), i32, name='G.sorted.rowmap')
+                lib.csr_permute_rows(s, M, nnz, self.G.rowPtrs.ptr, g_pk.ptr, rank8.ptr, int(padded.value),
                                      self.g_ptr.ptr, self.g_pk.ptr, self.g_map.ptr)
                 del rank8
-                # separable Kaiser-Bessel records in the same tile-sorted order: the forward gather then
-                # needs no stored entries at all (csrc/kbgrid.cu).  k-space between the two gridding steps is kept in this sorted order when both the separable
-                # forward gather and the x-run adjoint gather serve it: samples that are neighbours on the grid
-                # are then neighbours in memory (the original spoke order scatters them over 0.9 GB at cfg3)
-                self.kb = None
-                use_runs = self.allow_runs and C % 2 == 0 and self.tile[0] == 4 and kp % 4 == 0
-                use_tiles = self._want_tiles() is not None
+                # separable Kaiser-Bessel records in the same tile-sorted order: the forward gather then needs no
+                # stored entries at all (csrc/kbgrid.cu).  k-space between the two gridding steps is kept in this
+                # sorted order when both the separable forward gather and a sorted adjoint gather serve it: samples
+                # that are neighbours on the grid are then neighbours in memory (the original spoke order scatters
+                # them over 0.9 GB at cfg3)
+                use_runs, use_tiles = self.allow_runs and C % 2 == 0, self._want_tiles() is not None
                 self.ksp_sorted = bool(self.allow_separable and (use_runs or use_tiles) and self.allow_sorted_ksp)
                 if self.allow_separable:
-                    self.kb = kb_records_device(B, self.oN, coord, beta, weights, width, n, perm=self.g_map,
-                                                out_sorted=self.ksp_sorted)
+                    self.kb = kb_records_device(B, geo, coord, weights, perm=self.g_map, out_sorted=self.ksp_sorted)
                 if self.kb is None:
                     self.ksp_sorted = False
                 if self.ksp_sorted:
-                    self.pos = B.empty_array((max(self.M, 1),), i32, name='G.sorted.position')
-                    lib.invert_perm(s, self.M, self.g_map.ptr, self.pos.ptr)
+                    self.pos = B.empty_array((max(M, 1),), i32, name='G.sorted.position')
+                    lib.invert_perm(s, M, self.g_map.ptr, self.pos.ptr)
                 if self.kb is not None:
                     self.g_pk = self.g_ptr = None
             del g_pk
         # rows of G'^H that are long enough to deserve a whole CTA (k-space centre of radial trajectories)
         cnt = ctypes.c_int()
-        if not mf:
-            lib.csr_long_rows(s, kp, self.t_ptr.ptr, self.long_thresh, None, 0, ctypes.byref(cnt))
-        self.nlong, self.longrows = int(cnt.value), None
+        lib.csr_long_rows(s, kp, self.t_ptr.ptr, self.long_thresh, None, 0, ctypes.byref(cnt))
+        self.nlong = int(cnt.value)
         if self.nlong:
             self.longrows = B.empty_array((self.nlong,), i32, name='G.H.longrows')
             lib.csr_long_rows(s, kp, self.t_ptr.ptr, self.long_thresh, self.longrows.ptr, self.nlong, ctypes.byref(cnt))
-        # k-space support windows (csrc/kbgrid.cu, csrc/fft_pk.cuh): grid points no sample touches are neither
-        # written by the last forward pass, nor zero-filled by the adjoint gather, nor read by the first
-        # inverse pass.  Blocks of bx x 4 columns share one z interval; 16 interleaved lines (one FFT tile)
-        # must not straddle two blocks.
-        self.win, self.support_fraction = None, 1.0
-        if self.allow_windows and self.nnz and (C % 16 == 0 or 16 % C == 0):
-            bx = max(self.tile[0], 16 // C) if C < 16 else self.tile[0]
-            if self.oN[0] % bx == 0 and bx % self.tile[0] == 0:
-                win = B.empty_array((2 * self.oN[0] * self.oN[1],), i32, name='G.support')
-                rowmap_w = B.empty_array((kp,), i32, name='G.H.rowmap.support')
-                inside = ctypes.c_int64()
-                blk = (ctypes.c_int64 * 3)(bx, self.tile[1], self.tile[2])
-                if mf and self.kb is not None:
-                    lib.kb_support_windows(s, self.M, self.kb.ptr, grid3, kp, self.rowmap.ptr, blk, win.ptr, rowmap_w.ptr,
-                                           ctypes.byref(inside))
-                elif not mf:
-                    lib.grid_support_windows(s, grid3, kp, self.t_ptr.ptr, self.rowmap.ptr, blk, win.ptr, rowmap_w.ptr,
-                                             ctypes.byref(inside))
-                else:
-                    inside.value = self.on
-                frac = inside.value / float(self.on)
-                if frac <= 1.0 - self.window_min_saving:
-                    try:
-                        lib.sense_plan_set_support(self._plan, win.ptr, bx)
-                        self.win, self.rowmap, self.support_fraction = win, rowmap_w, frac
-                    except RuntimeError:
-                        pass                                            # geometry without persistent packed z passes
-        # block entries built from the separable records: one entry and one gather per (sample, block of 4 x by x bz
-        # grid points) pair -- whole tiles when the coils are few (the shard of a coil-sharded operator)
-        self.tiles = None
-        shape = self._want_tiles()
-        if self.real and self.kb is not None and shape:
-            from .sense import block_entries_device
-            by, bz = shape
-            t = block_entries_device(B, self.M, self.kb, self.oN, self.rowmap, kp, shape, self.tiles_seg_batches)
-            cl = 1
-            while cl < min(C, 16) // 2:
-                cl *= 2
-            t['scratch'] = B.empty_array((max(t['nslot'], 1) * 4 * by * bz * 2 * cl,), _C64, name='G.H.blocks.partial')
-            self.tiles = t
-        # x-run lists of the stored adjoint: one gather of a sample serves the four grid points of a tile row;
-        # runs longer than run_long_thresh entries are cut into segments with their own lane groups
-        self.runs = None
-        if not mf and self.tiles is None and self.real and self.allow_runs and C % 2 == 0 and self.tile[0] == 4 and kp % 4 == 0:
+        bx = self._window_block_x()
+        if bx:
+            win = B.empty_array((2 * self.oN[0] * self.oN[1],), i32, name='G.support')
+            rowmap_w = B.empty_array((kp,), i32, name='G.H.rowmap.support')
+            inside = ctypes.c_int64()
+            lib.grid_support_windows(s, (ctypes.c_int64 * 3)(*self.oN), kp, self.t_ptr.ptr, self.rowmap.ptr,
+                                     (ctypes.c_int64 * 3)(bx, GRID_TILE[1], GRID_TILE[2]), win.ptr, rowmap_w.ptr,
+                                     ctypes.byref(inside))
+            self._adopt_windows(win, rowmap_w, int(inside.value), bx)
+        if self.real and self.kb is not None and self._want_tiles() is not None:
+            self._build_blocks()
+            self.G = self.t_pk = self.t_ptr = self.t_val = self.t_ind = self.longrows = None
+            self.nlong = 0
+        elif self.real and self.allow_runs and C % 2 == 0:
+            # x-run lists of the stored adjoint: one gather of a sample serves the four grid points of a tile row;
+            # runs longer than run_long_thresh entries are cut into segments with their own lane groups
             seg = max(4, int(self.run_long_thresh) // 4 * 4)
             run_ptr = B.empty_array((kp // 4 + 1,), i32, name='G.H.runs.ptr')
             nre, nsg, nsp = ctypes.c_int64(), ctypes.c_int(), ctypes.c_int()
@@ -266,31 +223,47 @@ class SenseDevice(object):
             spld = B.empty_array((4 * max(nsp, 1),), i32, name='G.H.runs.split')
             lib.csr_runs_fill(s, kp, self.t_ptr.ptr, self.t_pk.ptr, seg, run_ptr.ptr, ids.ptr, w4.ptr, segd.ptr, spld.ptr,
                               self.pos.ptr if self.ksp_sorted else None)
-            cl = 1
-            while cl < C // 2:
-                cl *= 2
-            scratch = B.empty_array((max(nsg, 1) * 4 * 2 * cl,), _C64, name='G.H.runs.partial')
             self.runs = dict(ptr=run_ptr, ids=ids, w4=w4, seg=seg, segd=segd, nseg=nsg, spld=spld, nsplit=nsp,
-                             scratch=scratch, entries=int(nre.value))
-        # zero-initialised: with windows, parts of the grid are never written, and the separable gather
-        # multiplies its zero-weight taps (6th tap of on-grid samples) with whatever is there
-        if mf and (self.kb is None or self.tiles is None):
-            # the records or the block entries could not be built (kernel wider than 6 taps): construct on stored matrices
-            lib.sense_plan_destroy(self._plan)
-            self._plan = None
-            self.matrix_free_setup = False
-            return self.__init__(B, N, coord, maps, oversamp, weights, width, n)
-        if self.tiles is not None and self.kb is not None and not self.keep_stored:
-            # both gridding steps are matrix-free now: the CSR matrix, its stored adjoint and the long-row list were
-            # only the source of the support windows (17 GB at cfg3)
-            self.G = self.t_pk = self.t_ptr = self.t_val = self.t_ind = self.longrows = None
-            self.nlong = 0
-        self.grid = B.zero_array((self.on * C,), _C64, name='grid[z][y][x][c]')
-        self.ksp = B.empty_array((self.M * C,), _C64, name='ksp[m][c]')
+                             scratch=self._partial_sums(nsg, 4, C, 'G.H.runs.partial'), entries=int(nre.value))
+
+    def _window_block_x(self):
+        """x extent bx of the blocks of bx x 4 grid columns that share one support window (csrc/kbgrid.cu, fft_pk.cuh),
+        or None when windows do not apply: 16 interleaved lines (one FFT tile) must not straddle two blocks."""
+        C = self.C
+        if not (self.allow_windows and self.nnz and (C % 16 == 0 or 16 % C == 0)):
+            return None
+        bx = max(GRID_TILE[0], 16 // C)
+        return bx if self.oN[0] % bx == 0 else None
+
+    def _adopt_windows(self, win, rowmap_w, inside, bx):
+        """Let the passes and the adjoint gather skip the grid no sample touches, when that saves enough and the plan
+        allows it; rowmap_w then replaces the rowmap."""
+        frac = inside / float(self.on)
+        if frac <= 1.0 - self.window_min_saving:
+            try:
+                self.B._lib.sense_plan_set_support(self._plan, win.ptr, bx)
+                self.win, self.rowmap, self.support_fraction = win, rowmap_w, frac
+            except RuntimeError:
+                pass                                            # geometry without persistent packed z passes
+
+    def _build_blocks(self):
+        """Block entries from the separable records: one entry and one gather per (sample, block of 4 x by x bz grid
+        points) pair -- whole tiles when the coils are few (the shard of a coil-sharded operator)."""
+        by, bz = shape = self._want_tiles()
+        t = block_entries_device(self.B, self.M, self.kb, self.oN, self.rowmap, self.kp, shape, self.tiles_seg_batches)
+        t['scratch'] = self._partial_sums(t['nslot'], 4 * by * bz, min(self.C, 16), 'G.H.blocks.partial')
+        self.tiles = t
+
+    def _partial_sums(self, nslot, points, coils, name):
+        """Partial sums of nslot split work items of `points` grid points, one per pair of `coils` (power of two)."""
+        cl = 1
+        while cl < coils // 2:
+            cl *= 2
+        return self.B.empty_array((max(nslot, 1) * points * 2 * cl,), _C64, name=name)
 
     def _want_tiles(self):
         """Block shape (by, bz) of the matrix-free adjoint gather for this coil count, or None (x-runs / stored rows)."""
-        if not (self.allow_tiles and self.allow_separable and self.C % 2 == 0 and tuple(self.tile) == (4, 4, 4)):
+        if not (self.allow_tiles and self.allow_separable and self.C % 2 == 0):
             return None
         if self.block_shape:
             return tuple(self.block_shape)

@@ -10,9 +10,17 @@ After the -O3 recipe one `A.H * A` evaluation is the six backend calls of
 SURVEY.md section 3.1:
     ccsrmm(P^H, adjoint) -> fftn -> ccsrmm(G') -> ccsrmm(G', adjoint) -> ifftn -> ccsrmm(P^H)
 """
+import collections
+
 import numpy as np
 
 _C64 = np.dtype('complex64')
+
+# Tiles of the gridding structures of the fused operator and of the density compensation.  The adjoint gather's
+# kernels (block entries, x-runs) assume GRID_TILE = 4 x 4 x 4.
+SAMPLE_TILE = (8, 8, 8)     # samples are sorted by the grid tile of this size they fall into,
+SAMPLE_SUPER = (8, 8, 8)    # tiles grouped into super-tiles of this many tiles (64^3 points: L2-sized working set)
+GRID_TILE = (4, 4, 4)       # tile-major grid order: rows of the stored adjoint, blocks of the adjoint gather
 
 
 def _ops_of(B):
@@ -95,12 +103,11 @@ def _fftc_mod_times_scale(oN):
     (i_d - c_d/2) c_d/n_d) in float64 (backend.py:357-363) cast to complex64, times the
     complex64 cast of 1/sqrt(prod(oN)) (backend.py:349-351).  Evaluated slab by slab so
     that a 416^3 grid never needs the full float64 mgrid."""
-    n = int(np.prod(oN))
     terms = []
     for d in range(3):
         c = oN[d] // 2
         terms.append((np.arange(oN[d]) - c / 2.0) * (c / oN[d]))
-    scl = np.complex64(np.complex128(1.0) / np.sqrt(n))
+    scl = np.complex64(_grid_scale(oN))
     out = np.empty(oN, dtype=_C64, order='F')
     txy = (0 + terms[0][:, None]) + terms[1][None, :]
     for z in range(oN[2]):
@@ -135,22 +142,14 @@ def gridding_matrix_device(B, N, coord, oversamp=2.0, weights=None, width=3, n=1
     """G' = interp * (mod * scale) built on the GPU straight into device CSR arrays
     (ib200_kb_count -> exclusive scan -> ib200_kb_fill).  Returns (csr, oN, omin, beta).
     unphase (a unit constant u in {1, -1, i, -i}): build conj(u) * G' instead -- exact, and real when u is
-    _fftc_unit_phase(oN); the caller applies u through alpha."""
+    gridding_geometry(...).u; the caller applies u through alpha."""
     import ctypes
-    from scipy.signal.windows import kaiser
 
     lib, s = B._lib, B._stream
-    N = tuple(int(v) for v in N)
-    if isinstance(oversamp, tuple):
-        omin, os3 = min(oversamp), oversamp
-    else:
-        omin, os3 = oversamp, (oversamp,) * 3
-    oN = tuple(int(a * o) for a, o in zip(N, os3))
+    geo = gridding_geometry(N, oversamp, width, n)
+    oN, table = geo.oN, geo.table
     on = int(np.prod(oN))
-    beta = np.pi * np.sqrt(((width * 2. / omin) * (omin - 0.5)) ** 2 - 0.8)
-    table = np.ascontiguousarray(kaiser(2 * n + 1, beta)[n:], dtype=np.float64)
-    coord = np.asarray(coord)
-    c3 = np.asfortranarray(coord.reshape((3, -1), order='F').astype(np.float64))
+    c3 = _coords_f64(coord)
     m = c3.shape[1]
     grid = (ctypes.c_int64 * 3)(*oN)
     coord_d = B.copy_array(c3)
@@ -174,27 +173,28 @@ def gridding_matrix_device(B, N, coord, oversamp=2.0, weights=None, width=3, n=1
     B.barrier()
     del colscale_d, coord_d, counts
     Gd = B.csr_matrix.from_device(B, (m, on), g_ptr, g_ind[0:nnz], g_val[0:nnz], name='interp*mod*scale')
-    return Gd, oN, omin, beta
+    return Gd, oN, geo.omin, geo.beta
 
 
-def sample_order_device(B, oN, coord, width, tile, super_):
+def sample_order_device(B, geo, coord):
     """Matrix-free part of the fused operator's construction: (perm, nnz) with perm[r] = the sample at position r of
-    the tile-sorted order (ib200_kb_sample_order) and nnz = entries the gridding matrix would have (ib200_kb_count)."""
+    the tile-sorted order (ib200_kb_sample_order: SAMPLE_TILE tiles in SAMPLE_SUPER super-tiles) and nnz = entries
+    the gridding matrix would have (ib200_kb_count)."""
     import ctypes
     lib, s = B._lib, B._stream
-    c3 = np.asfortranarray(np.asarray(coord).reshape((3, -1), order='F').astype(np.float64))
+    c3 = _coords_f64(coord)
     m = c3.shape[1]
     coord_d = B.copy_array(c3)
-    grid = (ctypes.c_int64 * 3)(*oN)
+    grid = (ctypes.c_int64 * 3)(*geo.oN)
     i32 = np.dtype('int32')
     counts = B.empty_array((max(m, 1),), i32)
-    lib.kb_count(s, m, coord_d.ptr, grid, float(width), counts.ptr)
+    lib.kb_count(s, m, coord_d.ptr, grid, float(geo.width), counts.ptr)
     ptr = B.empty_array((m + 1,), i32)
     lib.exclusive_scan_i32(s, m, counts.ptr, ptr.ptr)
     nnz = int(ptr[m:m + 1].to_host()[0])
     perm = B.empty_array((max(m, 1),), i32, name='G.sorted.rowmap')
-    lib.kb_sample_order(s, m, coord_d.ptr, grid, float(width), (ctypes.c_int64 * 3)(*tile), (ctypes.c_int64 * 3)(*super_),
-                        perm.ptr)
+    lib.kb_sample_order(s, m, coord_d.ptr, grid, float(geo.width), (ctypes.c_int64 * 3)(*SAMPLE_TILE),
+                        (ctypes.c_int64 * 3)(*SAMPLE_SUPER), perm.ptr)
     return perm, nnz
 
 
@@ -215,65 +215,90 @@ def _fftc_unit_phases(oN):
     return out
 
 
-def _fftc_unit_phase(oN):
-    """Product of the per-axis unit constants (1 for every 3-D grid the fused path serves, -i for 2-D problems), or
-    None when the centring phase is not real up to a constant."""
+def _grid_scale(oN):
+    """The grid scale 1/sqrt(prod(oN)) as the -O2 realisation rounds it (complex64 cast, backend.py:349-351): a
+    float32."""
+    return np.float32(np.complex64(np.complex128(1.0) / np.sqrt(int(np.prod(oN)))).real)
+
+
+GriddingGeometry = collections.namedtuple('GriddingGeometry', 'N oN omin width beta table u factors separable')
+
+
+def gridding_geometry(N, oversamp=2.0, width=3, n=128):
+    """Oversampled grid and Kaiser-Bessel kernel of the NUFFT of an N image (backend.py:403-442): N, oN, omin (smallest
+    oversampling), width, beta, table (float64 right half of kaiser(2n + 1, beta)), u (unit constant of the centring
+    phase: 1 for every 3-D grid the fused path serves, -i for 2-D problems), factors (per-axis real factors of
+    conj(u) * mod * scale, float32, the scale folded into the last) and separable (whether ib200_kb_records can
+    describe G': at most 6 taps per axis).  When mod is not real up to a unit constant: u = 1, factors None."""
+    from scipy.signal.windows import kaiser
+    N = tuple(int(v) for v in N)
+    os3 = oversamp if isinstance(oversamp, tuple) else (oversamp,) * 3
+    oN = tuple(int(a * o) for a, o in zip(N, os3))
+    omin = min(os3)
+    beta = np.pi * np.sqrt(((width * 2. / omin) * (omin - 0.5)) ** 2 - 0.8)
+    table = np.ascontiguousarray(kaiser(2 * n + 1, beta)[n:], dtype=np.float64)
     ph = _fftc_unit_phases(oN)
-    if ph is None:
-        return None
-    u = complex(np.prod([p[0] for p in ph]))
-    return complex(round(u.real), round(u.imag))
+    u, factors = 1.0, None
+    if ph is not None:
+        u = complex(np.prod([p[0] for p in ph]))
+        u = complex(round(u.real), round(u.imag))
+        factors = [p[1] for p in ph]
+        factors[2] = (factors[2] * _grid_scale(oN)).astype(np.float32)
+    return GriddingGeometry(N, oN, omin, width, beta, table, u, factors,
+                            factors is not None and 2 * width <= 6)
 
 
-def _fftc_axis_factors(oN):
-    """Per-axis real factors of conj(u) * mod * scale (u = _fftc_unit_phase(oN)): three float32 arrays, the scale
-    folded into the last, or None when the centring phase is not real up to a constant."""
-    ph = _fftc_unit_phases(oN)
-    if ph is None:
-        return None
-    out = [p[1] for p in ph]
-    scl = np.float32(np.complex64(np.complex128(1.0) / np.sqrt(int(np.prod(oN)))).real)
-    out[2] = (out[2] * scl).astype(np.float32)
-    return out
+def _coords_f64(coord):
+    """Sample coordinates as the column-major float64 (3, M) array the construction kernels read; samples in the
+    order of coord.reshape((3, -1), order='F')."""
+    return np.asfortranarray(np.asarray(coord).reshape((3, -1), order='F').astype(np.float64))
 
 
-def kb_records_device(B, oN, coord, beta, weights=None, width=3, n=128, perm=None, out_sorted=False):
+def _mod_apod(geo):
+    """(cut, q): the image's window in the oversampled grid (Zpad 'center', backend.py:379-381) and q = mod * apod at
+    the image voxels, column-major complex64 (the diagonal factor of P, pics.py:111-126)."""
+    from .kbmath import rolloff3
+    cut = tuple(slice(a // 2 + int(np.ceil(-b / 2)), a // 2 + int(np.ceil(b / 2))) for a, b in zip(geo.oN, geo.N))
+    mod_at = _fftc_mod(geo.oN)[cut].flatten(order='F')
+    apod = rolloff3(geo.omin, geo.width, geo.beta, geo.N).flatten(order='F').astype(_C64)
+    return cut, (mod_at * np.complex64(1)) * apod
+
+
+def kb_records_device(B, geo, coord, weights=None, perm=None, out_sorted=False):
     """Separable-weight records of G' = interp*mod*scale (ib200_kb_records, csrc/kbgrid.cu): 96 bytes per
     sample instead of a stored row.  perm (device int32, optional): record r describes sample perm[r];
     out_sorted: results go to row r (sorted order) instead of row perm[r].
     Returns the device array of records, or None when this grid / kernel width is not served
-    (complex centring phase, more than 6 taps per axis)."""
+    (not geo.separable, or the kernel refuses a sample)."""
     import ctypes
-    from scipy.signal.windows import kaiser
 
-    fac = _fftc_axis_factors(oN)
-    if fac is None or 2 * width > 6:
+    if not geo.separable:
         return None
     lib, s = B._lib, B._stream
-    table = np.ascontiguousarray(kaiser(2 * n + 1, beta)[n:], dtype=np.float64)
-    c3 = np.asfortranarray(np.asarray(coord).reshape((3, -1), order='F').astype(np.float64))
+    c3 = _coords_f64(coord)
     m = c3.shape[1]
-    coord_d, table_d = B.copy_array(c3), B.copy_array(table)
-    f_d = [B.copy_array(np.ascontiguousarray(f)) for f in fac]
+    coord_d, table_d = B.copy_array(c3), B.copy_array(geo.table)
+    f_d = [B.copy_array(np.ascontiguousarray(f)) for f in geo.factors]
     w_d = None
     if weights is not None:
         w_d = B.copy_array(_sample_weights(weights, m))
     nb = int(lib.kb_record_bytes())
     rec = B.empty_array((max(m, 1) * nb // 8,), np.dtype('int64'), name='G.records')
     flag = ctypes.c_int()
-    grid = (ctypes.c_int64 * 3)(*oN)
-    lib.kb_records(s, m, coord_d.ptr, grid, float(width), table_d.ptr, int(table.size),
+    grid = (ctypes.c_int64 * 3)(*geo.oN)
+    lib.kb_records(s, m, coord_d.ptr, grid, float(geo.width), table_d.ptr, int(geo.table.size),
                    w_d.ptr if w_d is not None else None, f_d[0].ptr, f_d[1].ptr, f_d[2].ptr,
                    perm.ptr if perm is not None else None, 1 if out_sorted else 0, rec.ptr, ctypes.byref(flag))
     return rec if flag.value == 0 else None
 
 
-def tile_rowmap_device(B, oN, tile):
-    """Tile-major row order of the oversampled grid (ib200_grid_tile_rank): (kp, colrank, rowmap) with kp the padded
-    point count, colrank[point] its tile-major row and rowmap[row] the grid point of a row (< 0: padding)."""
+def tile_rowmap_device(B, oN):
+    """Tile-major row order of the oversampled grid in GRID_TILE tiles (ib200_grid_tile_rank): (kp, colrank, rowmap)
+    with kp the padded point count, colrank[point] its tile-major row and rowmap[row] the grid point of a row
+    (< 0: padding)."""
     import ctypes
     lib, s = B._lib, B._stream
-    grid3, tile3 = (ctypes.c_int64 * 3)(*oN), (ctypes.c_int64 * 3)(*tile)
+    grid3, tile3 = (ctypes.c_int64 * 3)(*oN), (ctypes.c_int64 * 3)(*GRID_TILE)
     padded = ctypes.c_int64()
     lib.grid_tile_rank(s, grid3, tile3, None, None, ctypes.byref(padded))
     kp = int(padded.value)
@@ -282,6 +307,23 @@ def tile_rowmap_device(B, oN, tile):
     rowmap = B.empty_array((kp,), i32, name='G.H.rowmap')
     lib.grid_tile_rank(s, grid3, tile3, colrank.ptr, rowmap.ptr, ctypes.byref(padded))
     return kp, colrank, rowmap
+
+
+def support_windows_device(B, m, records, oN, kp, rowmap, bx):
+    """k-space support windows from the separable records of m samples (ib200_kb_support_windows): one z interval
+    per column block of bx x GRID_TILE[1] grid points, the hull of the taps that fall into it.  Returns (win, rowmap_w,
+    inside): the windows, the tile-major rowmap of kp rows with the rows outside set to -1, and the number of grid
+    points inside."""
+    import ctypes
+    lib, s = B._lib, B._stream
+    i32 = np.dtype('int32')
+    win = B.empty_array((2 * oN[0] * oN[1],), i32, name='G.support')
+    rowmap_w = B.empty_array((kp,), i32, name='G.H.rowmap.support')
+    inside = ctypes.c_int64()
+    lib.kb_support_windows(s, m, records.ptr, (ctypes.c_int64 * 3)(*oN), kp, rowmap.ptr,
+                           (ctypes.c_int64 * 3)(bx, GRID_TILE[1], GRID_TILE[2]), win.ptr, rowmap_w.ptr,
+                           ctypes.byref(inside))
+    return win, rowmap_w, int(inside.value)
 
 
 def block_entries_device(B, m, records, oN, rowmap, kp, shape, seg_batches):
@@ -319,44 +361,34 @@ class DensityDevice(object):
 
     def __init__(self, B, N, coord, oversamp=2.0, width=3, n=128):
         import ctypes
-        from .fused import SenseDevice
         coord = np.asarray(coord)
         if not np.isfinite(coord).all():
             raise ValueError("pipe_menon_dcf: the trajectory has non-finite coordinates")
         self.B = B
-        lib, s = B._lib, B._stream
-        N = tuple(int(v) for v in N)
-        os3 = oversamp if isinstance(oversamp, tuple) else (oversamp,) * 3
-        oN = self.oN = tuple(int(a * o) for a, o in zip(N, os3))
-        omin = min(os3)
-        beta = np.pi * np.sqrt(((width * 2. / omin) * (omin - 0.5)) ** 2 - 0.8)       # as gridding_matrix_device
+        geo = gridding_geometry(N, oversamp, width, n)
+        oN = self.oN = geo.oN
         m = self.M = int(np.prod(coord.shape[1:]))
         self.shape = tuple(coord.shape[1:])
         self.grid3 = (ctypes.c_int64 * 3)(*oN)
-        self.perm, _ = sample_order_device(B, oN, coord, width, SenseDevice.sample_tile, SenseDevice.sample_super)
-        self.rec = kb_records_device(B, oN, coord, beta, None, width, n, perm=self.perm, out_sorted=True)
+        self.perm, _ = sample_order_device(B, geo, coord)
+        self.rec = kb_records_device(B, geo, coord, perm=self.perm, out_sorted=True)
         if self.rec is None:
             raise RuntimeError("pipe_menon_dcf: no separable records for kernel width %g on the oversampled grid %s "
                                "(they serve at most 6 taps per axis and a centring phase that is real up to a constant)"
                                % (width, oN))
-        kp, colrank, rowmap = tile_rowmap_device(B, oN, SenseDevice.tile)
+        kp, colrank, rowmap = tile_rowmap_device(B, oN)
         del colrank
-        i32 = np.dtype('int32')
-        win = B.empty_array((2 * oN[0] * oN[1],), i32, name='dcf.support')
-        self.rowmap = B.empty_array((kp,), i32, name='dcf.rowmap.support')
-        inside = ctypes.c_int64()
-        lib.kb_support_windows(s, m, self.rec.ptr, self.grid3, kp, rowmap.ptr, (ctypes.c_int64 * 3)(*SenseDevice.tile),
-                               win.ptr, self.rowmap.ptr, ctypes.byref(inside))
-        self.inside = int(inside.value)
+        win, self.rowmap, self.inside = support_windows_device(B, m, self.rec, oN, kp, rowmap, GRID_TILE[0])
         del win, rowmap
-        self.tiles = block_entries_device(B, m, self.rec, oN, self.rowmap, kp, (4, 4), SenseDevice.tiles_seg_batches)
+        # whole 4x4x4 tiles (one channel), blocks of more than 256 batches cut into work items
+        self.tiles = block_entries_device(B, m, self.rec, oN, self.rowmap, kp, (4, 4), 256)
         f32 = np.dtype('float32')
         self.scratch = B.empty_array((max(self.tiles['nslot'], 1) * 64,), f32, name='dcf.partial')
         self.g = B.zero_array((int(np.prod(oN)),), f32, name='dcf.grid')
         self.w = B.copy_array(np.ones(m, dtype=np.float32))
         self.resid = B.empty_array((1 + (m + 255) // 256,), np.dtype('float64'), name='dcf.residual')
         # the records carry scale = 1/sqrt(prod oN) (float32) on z: the update divides q = scale^2 (I I^T w) by it
-        scl = float(np.float32(np.complex64(np.complex128(1.0) / np.sqrt(int(np.prod(oN)))).real))
+        scl = float(_grid_scale(oN))
         self.inv_s2 = 1.0 / (scl * scl)
 
     def _step(self, label):
@@ -465,24 +497,17 @@ def sense_operator_device(B, N, coord, maps, oversamp=2.0, weights=None, width=3
     Needed at BASELINE.json's full sizes (416^3 grid, 6.8 M samples: 853 M stored entries).
     tests/test_gpu_sense.py checks structure (bit-identical) and values against the
     host-built matrices."""
-    import ctypes
-    from scipy.signal.windows import kaiser
-    from .kbmath import rolloff3
-
     lib, s = B._lib, B._stream
-    N = tuple(int(v) for v in N)
-    C = int(maps.shape[3])
-    Gd, oN, omin, beta = gridding_matrix_device(B, N, coord, oversamp, weights, width, n)
+    geo = gridding_geometry(N, oversamp, width, n)
+    N, oN, C = geo.N, geo.oN, int(maps.shape[3])
+    Gd = gridding_matrix_device(B, N, coord, oversamp, weights, width, n)[0]
     on, nvox = int(np.prod(oN)), int(np.prod(N))
 
     # ---- P^H, stored adjoint of kron(I_C, mod*zpad*apod) * vstack(maps) ----------------
-    cut = tuple(slice(a // 2 + int(np.ceil(-b / 2)), a // 2 + int(np.ceil(b / 2))) for a, b in zip(oN, N))
+    cut, q = _mod_apod(geo)                                                 # (mod @ zpad) @ apod
     lin = np.arange(on, dtype=np.int64).reshape(oN, order='F')
     zp = np.ascontiguousarray(lin[cut].flatten(order='F').astype(np.int32))
     del lin
-    mod_at = _fftc_mod(oN)[cut].flatten(order='F')
-    apod = rolloff3(omin, width, beta, N).flatten(order='F').astype(_C64)
-    q = np.ascontiguousarray((mod_at * np.complex64(1)) * apod)             # (mod @ zpad) @ apod
     maps_f = np.asfortranarray(maps.reshape((nvox, C), order='F').astype(_C64))
     maps_d, q_d, zp_d = B.copy_array(maps_f), B.copy_array(q), B.copy_array(zp)
     counts = B.empty_array((nvox,), np.dtype('int32'))
